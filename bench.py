@@ -2,7 +2,7 @@
 """Headline benchmark: exact top-10 QPS over a 10M x 1024 corpus (BASELINE.json configs[1]).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--workload cfg2|cfg3|cfg4|cfg5] [--rows R] [--batch B] [--k K]
+                    [--workload cfg2|cfg3|cfg4|cfg5] [--rows R] [--batch B] [--k K] [--dump-outputs DIR]
     torchrun --nproc-per-node N ... bench.py --gpus N ...          (one rank per GPU, NCCL)
 
 --workload selects the BASELINE.json configuration: cfg2 (default, the one the metric is quoted on: 10M x 1024,
@@ -22,6 +22,10 @@ host-buffer API (pinned host queries in, host results out, copies inside the tim
 scan kernel's algorithmic bytes / its CUDA-event time against the measured HBM copy peak; `cpu_baseline` = the
 numpy port of the reference's exact CPU scan on a bounded sample of the same workload; `parity` = the MERGED result
 the timed loop returned against the fp64 CPU oracle run over the whole corpus (rows read back from every shard).
+
+--dump-outputs DIR writes what the last timed step returned to its caller as DIR/rows.npy (global row ids, float64)
+and DIR/scores.npy (float32), one row per query of that batch.  Corpus and queries are seeded, so two builds run with
+the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -86,7 +90,11 @@ def parse():
     ap.add_argument("--no-cpu-parity", action="store_true", help="skip the CPU-oracle check over the whole corpus")
     ap.add_argument("--no-extras", action="store_true", help="skip the side measurements (batch1, batched, hybrid, cfg5)")
     ap.add_argument("--sustained-s", type=float, default=2.5)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy")
     a = ap.parse_args()
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs needs --impl ours: the reference arm scans a sample of the corpus")
     rows, batch, k = {"cfg2": (10_000_000, 64, 10), "cfg3": (10_000_000, 8192, 100), "cfg4": (5_000_000, 64, 10),
                       "cfg5": (100_000_000, 1024, 10)}[a.workload]
     a.rows = a.rows if a.rows is not None else rows
@@ -133,6 +141,25 @@ def peaks():
         return float(j["hbm_gbs"]), float(j.get("bf16_tflops_sustained", j["bf16_tflops"])), \
             "measured (MEASURED_PEAKS.json hbm_gbs / bf16_tflops_sustained)"
     return 6650.0, 1400.0, "fallback (B200_PROFILING.md)"
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(directory, arrays):
+    """arrays: name -> [B, ...] host array, one row per query.  Written as <directory>/<name>.npy, float32 arrays as
+    they are and everything else (row ids) as float64, which holds every row id exactly.  Above DUMP_LIMIT_BYTES in all,
+    a fixed seeded sample of the queries is written instead, their indices in query_index.npy."""
+    out = {n: np.asarray(v, dtype=np.float32 if v.dtype == np.float32 else np.float64) for n, v in arrays.items()}
+    n_queries = next(iter(out.values())).shape[0]
+    per_query = sum(v.nbytes for v in out.values()) // max(1, n_queries) + 8
+    if per_query * n_queries > DUMP_LIMIT_BYTES:
+        pick = np.sort(np.random.default_rng(0).choice(n_queries, DUMP_LIMIT_BYTES // per_query, replace=False))
+        out = {n: v[pick] for n, v in out.items()}
+        out["query_index"] = pick.astype(np.float64)
+    os.makedirs(directory, exist_ok=True)
+    for n, v in out.items():
+        np.save(os.path.join(directory, n + ".npy"), v)
 
 
 class ClockSampler:
@@ -404,6 +431,7 @@ class KnnLoop:
             t, i = tickets.pop(0)
             rows, scores = self.index.wait(t)
             self.account()
+            self.last = (rows, scores)          # the index's work buffers: valid until its next search
             if capture is not None and "rows" not in capture and capture["want"](i):
                 capture["rows"] = rows[:n_capture].clone()
                 capture["scores"] = scores[:n_capture].clone()
@@ -480,6 +508,8 @@ def run_ours(a):
     cap_main.pop("rows", None)
     cap_main.pop("scores", None)
     ms_dev, t0, t1 = loop.timed(step_dev, a.steps, 0, flush=flush_dev)
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, {"rows": loop.last[0].cpu().numpy(), "scores": loop.last[1].cpu().numpy()})
     stats = loop.stats
     scan_ms_avg = stats["scan_ms"] / max(1, stats["n"])
     bytes_per_step = stats["bytes"] / max(1, stats["n"])

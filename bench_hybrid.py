@@ -215,6 +215,7 @@ def measure(e, dev, csr, n_docs, B, steps, warmup, n_check, cpu_baseline=True, c
         return e0.elapsed_time(e1), t0, time.time()
 
     ms_dev, t0, t1 = timed(step_dev, steps, warmup, flush=finish)
+    last = {"rows": out_rows.cpu().numpy(), "scores": out_scores.cpu().numpy()}     # the fused lists of the last step
     dev_acc = dict(acc)
 
     # the text kernel's own duration: inside the pipelined loop its events also span the next batch's corpus pass (queued
@@ -244,7 +245,7 @@ def measure(e, dev, csr, n_docs, B, steps, warmup, n_check, cpu_baseline=True, c
            "text_only_kernel_ms": text_acc["text_ms"] / max(1, text_acc["n"]),
            "launches": int(dev_acc["launches"]), "order_free_batches": int(dev_acc["order_free"]),
            "mean_postings_per_query": float(np.mean(postings)) / B, "postings_per_batch": float(np.mean(postings)),
-           "term_bytes": int(np.mean([p[0].nbytes + p[1].nbytes for p in packed]))}
+           "term_bytes": int(np.mean([p[0].nbytes + p[1].nbytes for p in packed])), "last_outputs": last}
 
     # ---- parity against the CPU oracle at full size (test infrastructure, outside the timed region) ----
     if cpu_parity:
@@ -339,6 +340,8 @@ def run_ours(a, world, rank, dev):
     res = measure(e, dev, csr, n_docs, B, a.steps, a.warmup, 8, cpu_baseline=not a.no_cpu_baseline,
                   cpu_parity=not a.no_cpu_parity)
     sampler.stop()
+    if a.dump_outputs:
+        bench.dump_outputs(a.dump_outputs, res["last_outputs"])
     out = {"metric": "exact hybrid (BM25 multi_match + kNN fusion) top-10 QPS @5M chunks (ids identical to the CPU oracle)",
            "value": res["qps"], "unit": "queries/s", "n_gpus": 1, "steps": a.steps, "warmup": a.warmup,
            "ms_per_step": res["ms_dev"] / a.steps, "higher_is_better": True, "scaling": "strong", "vs_baseline": None,
