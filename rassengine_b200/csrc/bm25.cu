@@ -17,9 +17,6 @@
 
 #include "common.cuh"
 
-int search_core(rass_engine* h, const float* q_dev, int B, int k, int64_t* out_rows, float* out_scores,
-                double* out_keys, rass_stats* stats);
-
 template <typename T>
 static int upload(rass_engine* h, T** dst, const T* src, size_t n) {
   cudaFree(*dst);

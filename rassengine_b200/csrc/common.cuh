@@ -109,16 +109,50 @@ struct Bm25State {
   size_t scratch_bytes = 0;
 };
 
-// device-resident scalars the kernels update / read without a host round trip
-struct DevScalars {
+// device-resident facts of the store, raised by store_convert_kernel (atomicMax: they only ever grow), read by the
+// certificate of every search
+struct StoreScalars {
   float rho_x;        // max over rows of ||x - bf16(x)|| / ||x||
   float max_xnorm;    // max over rows of ||x||
+};
+
+// device-resident counters of one search, reset by query_prep_kernel
+struct SearchScalars {
   int flagged_n;      // queries that failed the certificate in the running search
   int max_cand;       // largest rerank candidate set in the running search
   int n_certified;
   int finish_done;    // CTAs of the running finish launch that are through (the last one publishes flagged_n, resets this)
   int tile_ctr[2];    // scan_umma_kernel's tile scheduler: tiles handed out beyond the first per CTA, CTAs through (the
                       // last one zeroes both)
+};
+
+// What one search in flight owns on the device (grows on demand).  The handle holds two: ws[0] serves the blocking
+// search and async slot 0, ws[1] async slot 1 under RASS_OPT_ASYNC_OVERLAP (allocated on its first use).
+struct SearchWs {
+  SearchScalars* scal = nullptr;    // device
+  // query workspace
+  int q_cap = 0;
+  float* q_raw = nullptr;           // [q_cap, dim_pad] fp32 as given (zero padded)
+  float* q_hat = nullptr;           // [q_cap, dim_pad] fp32 scan query (unit for cosine)
+  __nv_bfloat16* q16 = nullptr;     // [q_cap rounded to 64, dim_pad]
+  double* q_norm = nullptr;         // [q_cap]
+  float* q_rho = nullptr;           // [q_cap] ||q_hat - bf16(q_hat)|| / ||q_hat||
+  uint32_t* q_gthr = nullptr;       // [q_cap] tcgen05 scans: threshold seed, then the largest pivot any CTA published
+  // candidate pool of one query group (RASS_GROUP_Q queries)
+  size_t pool_entries = 0;          // per query: stride of the running search
+  size_t pool_alloc_entries = 0;    // allocated, in entries
+  float* pool_key = nullptr;
+  uint32_t* pool_row = nullptr;
+  size_t pool_segs = 0;             // per query: stride of the running search
+  size_t pool_alloc_segs = 0;       // allocated, in segments
+  float* pool_thr = nullptr;
+  int* pool_cnt = nullptr;
+  int* flagged = nullptr;           // device [q_cap]: ids of queries that failed the certificate
+  int* flagged_host = nullptr;      // pinned [q_cap]
+  void* tmap_q = nullptr;           // host copy of the CUtensorMap over q16, 64-row boxes (scan_umma)
+  void* tmap_q2 = nullptr;          // 128-row boxes (scan_gemm: one CTA's half of a 256-query group)
+  const void* tmap_qbase = nullptr; // the q16 each map was encoded for
+  const void* tmap_q2base = nullptr;
 };
 
 // a device array that grows in place (vmm.cu): reserved address range, physical chunks mapped on demand
@@ -150,8 +184,9 @@ struct rass_engine {
   // pointer); otherwise they are cudaMalloc'ed and grow by copy
   VmArray vm[5];
   bool use_vm = false;
-  DevScalars* scal = nullptr;       // device
-  DevScalars* scal_host = nullptr;  // pinned mirror
+  StoreScalars* store_scal = nullptr;   // device
+  SearchWs ws[2];
+  SearchScalars* scal_host = nullptr;   // pinned mirror of ws[0].scal for the blocking search
   cudaStream_t stream = nullptr, user_stream = nullptr, copy_stream = nullptr;
   bool has_user_stream = false;     // user_stream may legitimately be 0 (the legacy default stream)
   cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
@@ -160,29 +195,10 @@ struct rass_engine {
   size_t stage_bytes = 0;
   float* dev_stage = nullptr;            // device staging (BF16_ONLY appends, dim != dim_pad appends)
   size_t dev_stage_bytes = 0;
-  // query workspace (grows on demand)
-  int q_cap = 0;
-  float* q_raw = nullptr;           // [q_cap, dim_pad] fp32 as given (zero padded)
-  float* q_hat = nullptr;           // [q_cap, dim_pad] fp32 scan query (unit for cosine)
-  __nv_bfloat16* q16 = nullptr;     // [q_cap rounded to 64, dim_pad]
-  double* q_norm = nullptr;         // [q_cap]
-  float* q_rho = nullptr;           // [q_cap] ||q_hat - bf16(q_hat)|| / ||q_hat||
-  uint32_t* q_gthr = nullptr;       // [q_cap] tcgen05 scans: threshold seed, then the largest pivot any CTA published
-  // candidate pool of one query group (RASS_GROUP_Q queries)
-  size_t pool_entries = 0;          // per query: stride of the running search
-  size_t pool_alloc_entries = 0;    // allocated, in entries
-  float* pool_key = nullptr;
-  uint32_t* pool_row = nullptr;
-  size_t pool_segs = 0;             // per query: stride of the running search
-  size_t pool_alloc_segs = 0;       // allocated, in segments
-  float* pool_thr = nullptr;
-  int* pool_cnt = nullptr;
   // exact (fp64) lists
   size_t xlist_entries = 0;
   double* xlist_key = nullptr;
   uint32_t* xlist_row = nullptr;
-  int* flagged = nullptr;           // device [q_cap]: ids of queries that failed the certificate
-  int* flagged_host = nullptr;      // pinned [q_cap]
   int64_t* out_rows = nullptr;      // device result staging for the host-pointer API
   float* out_scores = nullptr;
   double* out_keys = nullptr;
@@ -196,12 +212,8 @@ struct rass_engine {
   std::vector<uint8_t> dead;        // host mirror of the tombstones
   std::vector<cudaEvent_t> ev_pool; // per-group scan timing
   void* tmap_x = nullptr;           // host copy of the CUtensorMap over x16 (rebuilt on growth)
-  void* tmap_q = nullptr;           // queries, 64-row boxes (scan_umma)
-  void* tmap_q2 = nullptr;          // queries, 128-row boxes (scan_gemm: one CTA's half of a 256-query group)
-  const void* tmap_q2base = nullptr;
   int64_t tmap_rows = -1;
   const void* tmap_base = nullptr;
-  const void* tmap_qbase = nullptr;
   // second-chance pass (queries whose certificate failed at k > 32): ids, gathered queries, results
   int* retry_ids = nullptr;
   float* retry_q = nullptr;
@@ -211,37 +223,16 @@ struct rass_engine {
   size_t retry_cap = 0;
   int retry_k = 0;
   // RASS_OPT_ASYNC_OVERLAP: each async slot runs on its own stream (forked from the engine stream when the search is
-  // enqueued) and slot 1 owns a second search workspace, so the fixed costs of batch i (query prep, threshold seed,
-  // finish) run under the scan of batch i+1.  While slot 1's search is being enqueued the workspace fields of the handle
-  // are swapped with `ws_alt` (kernels capture the pointers at launch).
-  struct SearchWs {
-    DevScalars* scal = nullptr;
-    int q_cap = 0;
-    float *q_raw = nullptr, *q_hat = nullptr;
-    __nv_bfloat16* q16 = nullptr;
-    double* q_norm = nullptr;
-    float* q_rho = nullptr;
-    uint32_t* q_gthr = nullptr;
-    size_t pool_entries = 0, pool_alloc_entries = 0;
-    float* pool_key = nullptr;
-    uint32_t* pool_row = nullptr;
-    size_t pool_segs = 0, pool_alloc_segs = 0;
-    float* pool_thr = nullptr;
-    int* pool_cnt = nullptr;
-    int *flagged = nullptr, *flagged_host = nullptr;
-    void *tmap_q = nullptr, *tmap_q2 = nullptr;
-    const void *tmap_q2base = nullptr, *tmap_qbase = nullptr;
-  } ws_alt;
+  // enqueued) and slot 1 uses the second search workspace ws[1], so the fixed costs of batch i (query prep, threshold
+  // seed, finish) run under the scan of batch i+1.
   bool async_overlap = false;
   int scan_reserve_sms = 0;         // RASS_OPT_SCAN_RESERVE_SMS
   cudaStream_t slot_stream[2] = {nullptr, nullptr};
   cudaEvent_t slot_fork[2] = {nullptr, nullptr};
-  uint64_t store_version = 1;       // bumped whenever rho_x / max_xnorm may have changed (store_convert launches)
-  uint64_t alt_store_version = 0;   // the version ws_alt.scal mirrors
   // two searches may be in flight through rass_search_knn_dev_async (one slot each)
   struct AsyncSlot {
     bool pending = false, trivial = false;
-    DevScalars* scal_host = nullptr;   // pinned
+    SearchScalars* scal_host = nullptr;   // pinned: its own copy, a blocking search may reuse ws[0] before the wait
     cudaEvent_t done = nullptr;
     size_t n_ev = 0;
     rass_stats stats;
@@ -280,7 +271,6 @@ static inline cudaStream_t eng_stream(const rass_engine* h) { return h->has_user
 static inline cudaStream_t slot_stream_of(const rass_engine* h, int slot) {
   return h->async_overlap && h->slot_stream[slot] ? h->slot_stream[slot] : eng_stream(h);
 }
-void swap_search_ws(rass_engine* h);
 
 // fp32 accumulation allowance of a length-d dot product with |x||q| <= 1 (gamma_d, doubled for the tensor
 // pipe's unspecified summation order)
@@ -510,35 +500,37 @@ __device__ __forceinline__ float score_from_key(double key, int metric) {
 // ---------------------------------------------------------------------------------------------
 int launch_store_convert(rass_engine* h, const float* src_dev, int64_t src_stride, int64_t first_row, int64_t n,
                          cudaStream_t st);
-int launch_query_prep(rass_engine* h, const float* q_dev, int B, cudaStream_t st);
-int launch_seed_thresholds(rass_engine* h, int B, int seg, size_t n_clear, bool* cleared, cudaStream_t st);
+int launch_query_prep(rass_engine* h, const SearchWs& ws, const float* q_dev, int B, cudaStream_t st);
+int launch_seed_thresholds(rass_engine* h, const SearchWs& ws, int B, int seg, size_t n_clear, bool* cleared,
+                           cudaStream_t st);
 // streaming scan of queries [q0, q0+nq) (nq = 1 or 2); their pool slots are q - g0
-int launch_scan_stream(rass_engine* h, int q0, int nq, int g0, cudaStream_t st);
+int launch_scan_stream(rass_engine* h, const SearchWs& ws, int q0, int nq, int g0, cudaStream_t st);
 int scan_stream_segs(const rass_engine* h);
 // tcgen05 scan of queries [q0, q0+nq) (nq <= 64) into pool slots 0..nq
-int launch_scan_umma(rass_engine* h, int q0, int nq, int seg, cudaStream_t st, bool pool_cleared = false);
+int launch_scan_umma(rass_engine* h, SearchWs& ws, int q0, int nq, int seg, cudaStream_t st, bool pool_cleared = false);
 int scan_umma_segs(const rass_engine* h);
-int umma_selftest(rass_engine* h, int n_rows_tile, float* out_host, cudaStream_t st);
+int umma_selftest(rass_engine* h, SearchWs& ws, int n_rows_tile, float* out_host, cudaStream_t st);
 // CTA-pair tcgen05 scan of all B prepared queries (groups of 256) into pool slots 0..B
-int launch_scan_gemm(rass_engine* h, int B, int seg, cudaStream_t st, bool pool_cleared = false);
+int launch_scan_gemm(rass_engine* h, SearchWs& ws, int B, int seg, cudaStream_t st, bool pool_cleared = false);
 int scan_gemm_segs(const rass_engine* h, int B);
-int gemm_selftest(rass_engine* h, int B, float* out_host, cudaStream_t st);
+int gemm_selftest(rass_engine* h, SearchWs& ws, int B, float* out_host, cudaStream_t st);
 // CUtensorMap over a [rows, dim_pad] bf16 matrix: boxes of box_rows x 64 elements, 128B swizzle
 int encode_rows_map(rass_engine* h, void* map, const void* base, int64_t rows, int box_rows);
 // merge the pool of queries [g0, g0+ng), rerank in fp64, emit top-k, flag uncertified queries
-int launch_finish(rass_engine* h, int g0, int ng, int k, int n_segs, int seg_size, bool has_cnt, bool q_is_bf16,
-                  int64_t* out_rows, float* out_scores, double* out_keys, cudaStream_t st,
+int launch_finish(rass_engine* h, const SearchWs& ws, int g0, int ng, int k, int n_segs, int seg_size, bool has_cnt,
+                  bool q_is_bf16, int64_t* out_rows, float* out_scores, double* out_keys, cudaStream_t st,
                   int64_t* flag_out = nullptr);
 // fp64 scan of the listed queries (qids host array, n_q of them)
-int launch_exact(rass_engine* h, int k, const int* qids_host, int n_q, int64_t* out_rows, float* out_scores,
-                 double* out_keys, cudaStream_t st, int* launches);
+int launch_exact(rass_engine* h, const SearchWs& ws, int k, const int* qids_host, int n_q, int64_t* out_rows,
+                 float* out_scores, double* out_keys, cudaStream_t st, int* launches);
 // raw_score: the keys are fused scores (larger is better whatever the engine's metric), emitted as they are
 int launch_merge_topk(rass_engine* h, const double* keys, const int64_t* rows, int64_t shard_stride, int G, int B,
                       int k, int64_t* out_rows, float* out_scores, double* out_keys, cudaStream_t st,
                       bool raw_score = false);
-// blocking (async_slot < 0) or enqueue-only search of prepared device queries (engine.cu)
-int search_core_ex(rass_engine* h, const float* q_dev, int B, int k, int64_t* out_rows, float* out_scores,
-                   double* out_keys, rass_stats* stats, int async_slot, int64_t* async_flag_dev);
+// kNN search of B device queries [B, dim] fp32 into device outputs (engine.cu): blocking (async_slot < 0, the stream
+// is synchronised before returning) or enqueue-only into async slot 0 / 1 (rass_search_knn_dev_async)
+int search_core(rass_engine* h, const float* q_dev, int B, int k, int64_t* out_rows, float* out_scores,
+                double* out_keys, rass_stats* stats, int async_slot = -1, int64_t* async_flag_dev = nullptr);
 int stage_queries(rass_engine* h, const float* q_host, int B, float** q_dev_out);
 // Row-sharded hybrid: fuse against an EXTERNAL (global) knn list and leave this shard's top-k on the device
 struct HybridExt {
@@ -619,7 +611,8 @@ rass_engine* sharded_first(rass_engine* h);      // the shard on the coordinator
     if ((h) && (h)->shards) return call; \
   } while (0)
 
-int ensure_query_workspace(rass_engine* h, int B);
-int ensure_pool(rass_engine* h, size_t entries_per_query, size_t segs_per_query, size_t n_queries = RASS_GROUP_Q);
+int ensure_query_workspace(rass_engine* h, SearchWs& ws, int B);
+int ensure_pool(rass_engine* h, SearchWs& ws, size_t entries_per_query, size_t segs_per_query,
+                size_t n_queries = RASS_GROUP_Q);
 int ensure_xlist_workspace(rass_engine* h, size_t entries);
 int ensure_out_workspace(rass_engine* h, size_t n);

@@ -160,10 +160,12 @@ extern "C" int rass_create(int dim, int metric, int device, int64_t capacity_row
   for (int i = 0; i < 2; ++i) CREATE_TRY(cudaEventCreateWithFlags(&h->stage_ev[i], cudaEventDisableTiming));
   h->stage_bytes = (size_t)32 << 20;
   for (int i = 0; i < 2; ++i) CREATE_TRY(cudaMallocHost(&h->stage[i], h->stage_bytes));
-  CREATE_TRY(cudaMalloc(&h->scal, sizeof(DevScalars)));
-  CREATE_TRY(cudaMemset(h->scal, 0, sizeof(DevScalars)));
-  CREATE_TRY(cudaMallocHost(&h->scal_host, sizeof(DevScalars)));
-  memset(h->scal_host, 0, sizeof(DevScalars));
+  CREATE_TRY(cudaMalloc(&h->store_scal, sizeof(StoreScalars)));
+  CREATE_TRY(cudaMemset(h->store_scal, 0, sizeof(StoreScalars)));
+  CREATE_TRY(cudaMalloc(&h->ws[0].scal, sizeof(SearchScalars)));
+  CREATE_TRY(cudaMemset(h->ws[0].scal, 0, sizeof(SearchScalars)));
+  CREATE_TRY(cudaMallocHost(&h->scal_host, sizeof(SearchScalars)));
+  memset(h->scal_host, 0, sizeof(SearchScalars));
 #undef CREATE_TRY
   if (capacity_rows > 0) {
     int rc = ensure_capacity(h, capacity_rows);
@@ -171,6 +173,14 @@ extern "C" int rass_create(int dim, int metric, int device, int64_t capacity_row
   }
   *out = h;
   return RASS_OK;
+}
+
+static void free_search_ws(SearchWs& w) {
+  cudaFree(w.scal);
+  cudaFree(w.q_raw); cudaFree(w.q_hat); cudaFree(w.q16); cudaFree(w.q_norm); cudaFree(w.q_rho); cudaFree(w.q_gthr);
+  cudaFree(w.pool_key); cudaFree(w.pool_row); cudaFree(w.pool_thr); cudaFree(w.pool_cnt);
+  cudaFree(w.flagged); cudaFreeHost(w.flagged_host);
+  free(w.tmap_q); free(w.tmap_q2);
 }
 
 extern "C" int rass_destroy(rass_engine* h) {
@@ -183,12 +193,10 @@ extern "C" int rass_destroy(rass_engine* h) {
   } else {
     cudaFree(h->x32); cudaFree(h->x16); cudaFree(h->norm64); cudaFree(h->sa); cudaFree(h->sb);
   }
-  cudaFree(h->scal); cudaFreeHost(h->scal_host);
+  cudaFree(h->store_scal); cudaFreeHost(h->scal_host);
+  for (SearchWs& w : h->ws) free_search_ws(w);
   cudaFree(h->dev_stage);
-  cudaFree(h->q_raw); cudaFree(h->q_hat); cudaFree(h->q16); cudaFree(h->q_norm); cudaFree(h->q_rho); cudaFree(h->q_gthr);
-  cudaFree(h->pool_key); cudaFree(h->pool_row); cudaFree(h->pool_thr); cudaFree(h->pool_cnt);
   cudaFree(h->xlist_key); cudaFree(h->xlist_row);
-  cudaFree(h->flagged); cudaFreeHost(h->flagged_host);
   cudaFree(h->out_rows); cudaFree(h->out_scores); cudaFree(h->out_keys);
   cudaFreeHost(h->out_rows_host); cudaFreeHost(h->out_scores_host); cudaFreeHost(h->out_keys_host);
   cudaFreeHost(h->q_stage_host);
@@ -198,14 +206,6 @@ extern "C" int rass_destroy(rass_engine* h) {
   cudaFree(h->flist_dev);
   cudaFree(h->sb_filtered);
   cudaFree(h->retry_ids); cudaFree(h->retry_q); cudaFree(h->retry_rows); cudaFree(h->retry_scores); cudaFree(h->retry_keys);
-  {
-    rass_engine::SearchWs& w = h->ws_alt;
-    cudaFree(w.scal);
-    cudaFree(w.q_raw); cudaFree(w.q_hat); cudaFree(w.q16); cudaFree(w.q_norm); cudaFree(w.q_rho); cudaFree(w.q_gthr);
-    cudaFree(w.pool_key); cudaFree(w.pool_row); cudaFree(w.pool_thr); cudaFree(w.pool_cnt);
-    cudaFree(w.flagged); cudaFreeHost(w.flagged_host);
-    free(w.tmap_q); free(w.tmap_q2);
-  }
   for (int i = 0; i < 2; ++i) {
     if (h->slot_stream[i]) cudaStreamDestroy(h->slot_stream[i]);
     if (h->slot_fork[i]) cudaEventDestroy(h->slot_fork[i]);
@@ -222,7 +222,7 @@ extern "C" int rass_destroy(rass_engine* h) {
   cudaFree(b.gen_dev);
   cudaFree(b.scratch);
   cudaFree(b.vocab_blob); cudaFree(b.vocab_off); cudaFree(b.fz_terms); cudaFree(b.fz_edits); cudaFree(b.fz_n);
-  free(h->tmap_x); free(h->tmap_q); free(h->tmap_q2);
+  free(h->tmap_x);
   if (h->stream) cudaStreamDestroy(h->stream);
   if (h->copy_stream) cudaStreamDestroy(h->copy_stream);
   delete h;
@@ -587,68 +587,42 @@ static int sync_for_realloc(rass_engine* h) {
   return RASS_OK;
 }
 
-void swap_search_ws(rass_engine* h) {
-  rass_engine::SearchWs& w = h->ws_alt;
-  std::swap(h->scal, w.scal);
-  std::swap(h->q_cap, w.q_cap);
-  std::swap(h->q_raw, w.q_raw);
-  std::swap(h->q_hat, w.q_hat);
-  std::swap(h->q16, w.q16);
-  std::swap(h->q_norm, w.q_norm);
-  std::swap(h->q_rho, w.q_rho);
-  std::swap(h->q_gthr, w.q_gthr);
-  std::swap(h->pool_entries, w.pool_entries);
-  std::swap(h->pool_alloc_entries, w.pool_alloc_entries);
-  std::swap(h->pool_key, w.pool_key);
-  std::swap(h->pool_row, w.pool_row);
-  std::swap(h->pool_segs, w.pool_segs);
-  std::swap(h->pool_alloc_segs, w.pool_alloc_segs);
-  std::swap(h->pool_thr, w.pool_thr);
-  std::swap(h->pool_cnt, w.pool_cnt);
-  std::swap(h->flagged, w.flagged);
-  std::swap(h->flagged_host, w.flagged_host);
-  std::swap(h->tmap_q, w.tmap_q);
-  std::swap(h->tmap_q2, w.tmap_q2);
-  std::swap(h->tmap_q2base, w.tmap_q2base);
-  std::swap(h->tmap_qbase, w.tmap_qbase);
-}
-
-int ensure_query_workspace(rass_engine* h, int B) {
-  if (B <= h->q_cap) return RASS_OK;
+int ensure_query_workspace(rass_engine* h, SearchWs& ws, int B) {
+  if (B <= ws.q_cap) return RASS_OK;
   { const int rc_ = sync_for_realloc(h); if (rc_) return rc_; }
   const size_t cap = (size_t)(B + RASS_QPAD - 1) / RASS_QPAD * RASS_QPAD, d = (size_t)h->dim_pad;
-  REALLOC_DEV(h, h->q_raw, cap * d);
-  REALLOC_DEV(h, h->q_hat, cap * d);
-  REALLOC_DEV(h, h->q16, cap * d);
-  REALLOC_DEV(h, h->q_norm, cap);
-  REALLOC_DEV(h, h->q_rho, cap);
-  REALLOC_DEV(h, h->q_gthr, cap);
-  REALLOC_DEV(h, h->flagged, cap);
-  REALLOC_HOST(h, h->flagged_host, cap);
-  h->q_cap = (int)cap;
-  h->tmap_qbase = nullptr;
-  h->tmap_q2base = nullptr;
+  REALLOC_DEV(h, ws.q_raw, cap * d);
+  REALLOC_DEV(h, ws.q_hat, cap * d);
+  REALLOC_DEV(h, ws.q16, cap * d);
+  REALLOC_DEV(h, ws.q_norm, cap);
+  REALLOC_DEV(h, ws.q_rho, cap);
+  REALLOC_DEV(h, ws.q_gthr, cap);
+  REALLOC_DEV(h, ws.flagged, cap);
+  REALLOC_HOST(h, ws.flagged_host, cap);
+  ws.q_cap = (int)cap;
+  ws.tmap_qbase = nullptr;
+  ws.tmap_q2base = nullptr;
   return RASS_OK;
 }
 
-int ensure_pool(rass_engine* h, size_t entries_per_query, size_t segs_per_query, size_t n_queries) {
+int ensure_pool(rass_engine* h, SearchWs& ws, size_t entries_per_query, size_t segs_per_query, size_t n_queries) {
   const size_t need_e = entries_per_query * n_queries, need_s = segs_per_query * n_queries;
-  if (need_e > h->pool_alloc_entries) {
+  if (need_e > ws.pool_alloc_entries) {
     { const int rc_ = sync_for_realloc(h); if (rc_) return rc_; }
-    h->pool_alloc_entries = 0;
-    REALLOC_DEV(h, h->pool_key, need_e);
-    REALLOC_DEV(h, h->pool_row, need_e);
-    h->pool_alloc_entries = need_e;
+    ws.pool_alloc_entries = 0;
+    REALLOC_DEV(h, ws.pool_key, need_e);
+    REALLOC_DEV(h, ws.pool_row, need_e);
+    ws.pool_alloc_entries = need_e;
   }
-  if (need_s > h->pool_alloc_segs) {
+  if (need_s > ws.pool_alloc_segs) {
     { const int rc_ = sync_for_realloc(h); if (rc_) return rc_; }
-    h->pool_alloc_segs = 0;
-    REALLOC_DEV(h, h->pool_thr, need_s);
-    REALLOC_DEV(h, h->pool_cnt, need_s);
-    h->pool_alloc_segs = need_s;
+    ws.pool_alloc_segs = 0;
+    REALLOC_DEV(h, ws.pool_thr, need_s);
+    REALLOC_DEV(h, ws.pool_cnt, need_s);
+    ws.pool_alloc_segs = need_s;
   }
-  h->pool_entries = entries_per_query;
-  h->pool_segs = segs_per_query;
+  ws.pool_entries = entries_per_query;
+  ws.pool_segs = segs_per_query;
   return RASS_OK;
 }
 
@@ -749,20 +723,16 @@ __global__ void scatter_results_kernel(const int* __restrict__ ids, int k, const
   }
 }
 
-static int search_core_impl(rass_engine* h, const float* q_dev, int B, int k, int64_t* out_rows, float* out_scores,
-                            double* out_keys, rass_stats* stats, bool robust, int async_slot = -1,
-                            int64_t* async_flag_dev = nullptr);
-
-// q_dev: [B, dim] fp32 on this device; outputs on this device.  Synchronises the stream before returning.
-int search_core(rass_engine* h, const float* q_dev, int B, int k, int64_t* out_rows, float* out_scores,
-                double* out_keys, rass_stats* stats) {
-  return search_core_impl(h, q_dev, B, k, out_rows, out_scores, out_keys, stats, false, -1, nullptr);
-}
-
-// the same with the async form exposed (sharded.cu drives one of these per shard)
-int search_core_ex(rass_engine* h, const float* q_dev, int B, int k, int64_t* out_rows, float* out_scores,
-                   double* out_keys, rass_stats* stats, int async_slot, int64_t* async_flag_dev) {
-  return search_core_impl(h, q_dev, B, k, out_rows, out_scores, out_keys, stats, false, async_slot, async_flag_dev);
+// the scan time of a search: the sum over its pairs of timing events (ev_pool[base + i], ev_pool[base + i + 1])
+static int scan_ms_of(rass_engine* h, size_t base, size_t n_ev, double* out) {
+  double ms = 0.0;
+  for (size_t i = 0; i + 1 < n_ev; i += 2) {
+    float t = 0.f;
+    CUDA_TRY(h, cudaEventElapsedTime(&t, h->ev_pool[base + i], h->ev_pool[base + i + 1]));
+    ms += t;
+  }
+  *out = ms;
+  return RASS_OK;
 }
 
 // robust = false: 256-entry segments (a compaction keeps 32..64 entries): fastest, and every pivot has >= 32 >= k
@@ -772,62 +742,11 @@ int search_core_ex(rass_engine* h, const float* q_dev, int B, int k, int64_t* ou
 //
 // async_slot >= 0: enqueue only -- no host synchronisation, no fallback; the certificate outcome lands in the slot's
 // pinned scalars (and, for row-sharded callers, in *async_flag_dev, which travels with the all-gathered candidates).
-static int search_core_body(rass_engine* h, const float* q_dev, int B, int k, int64_t* out_rows, float* out_scores,
-                            double* out_keys, rass_stats* stats, bool robust, int async_slot, int64_t* async_flag_dev,
-                            cudaStream_t st);
-
-static int search_core_impl(rass_engine* h, const float* q_dev, int B, int k, int64_t* out_rows, float* out_scores,
-                            double* out_keys, rass_stats* stats, bool robust, int async_slot, int64_t* async_flag_dev) {
-  if (B < 1) return rass_fail(h, RASS_E_INVALID, "B must be >= 1");
-  if (k < 1 || k > RASS_MAX_K) return rass_fail(h, RASS_E_INVALID, "k must be in [1, %d], got %d", RASS_MAX_K, k);
-  cudaStream_t st = eng_stream(h);
+static int search_core_body(rass_engine* h, SearchWs& ws, const float* q_dev, int B, int k, int64_t* out_rows,
+                            float* out_scores, double* out_keys, rass_stats* stats, bool robust, int async_slot,
+                            int64_t* async_flag_dev, cudaStream_t st) {
   int rc;
-  if (!h->async_overlap)
-    return search_core_body(h, q_dev, B, k, out_rows, out_scores, out_keys, stats, robust, async_slot, async_flag_dev, st);
-  if (async_slot < 0) {
-    // a blocking search shares slot 0's workspace (and must see everything enqueued so far): order it behind the
-    // searches in flight
-    for (auto& a : h->aslot)
-      if (a.pending && a.done) CUDA_TRY(h, cudaStreamWaitEvent(st, a.done, 0));
-    return search_core_body(h, q_dev, B, k, out_rows, out_scores, out_keys, stats, robust, async_slot, async_flag_dev, st);
-  }
-  if (h->aslot[async_slot].pending)
-    return rass_fail(h, RASS_E_INVALID, "async slot %d still has a search in flight", async_slot);
-  if (!h->slot_stream[async_slot]) {
-    CUDA_TRY(h, cudaStreamCreateWithFlags(&h->slot_stream[async_slot], cudaStreamNonBlocking));
-    CUDA_TRY(h, cudaEventCreateWithFlags(&h->slot_fork[async_slot], cudaEventDisableTiming));
-  }
-  // the folded filter offsets are shared by both slots: (re)build them ahead of the fork, on the engine stream
-  if ((rc = select_scan_offsets(h, st))) return rc;
-  cudaStream_t ss = h->slot_stream[async_slot];
-  CUDA_TRY(h, cudaEventRecord(h->slot_fork[async_slot], st));
-  CUDA_TRY(h, cudaStreamWaitEvent(ss, h->slot_fork[async_slot], 0));
-  if (async_slot == 0)
-    return search_core_body(h, q_dev, B, k, out_rows, out_scores, out_keys, stats, robust, async_slot, async_flag_dev, ss);
-  swap_search_ws(h);
-  rc = RASS_OK;
-  if (!h->scal) {
-    cudaError_t e = cudaMalloc(&h->scal, sizeof(DevScalars));
-    if (e == cudaSuccess) e = cudaMemsetAsync(h->scal, 0, sizeof(DevScalars), ss);
-    if (e != cudaSuccess) rc = rass_fail(h, RASS_E_CUDA, "second search workspace: %s", cudaGetErrorString(e));
-    h->alt_store_version = 0;
-  }
-  if (!rc && h->alt_store_version != h->store_version) {       // rho_x / max_xnorm of the store, as of this search
-    cudaError_t e = cudaMemcpyAsync(h->scal, h->ws_alt.scal, 2 * sizeof(float), cudaMemcpyDeviceToDevice, ss);
-    if (e != cudaSuccess) rc = rass_fail(h, RASS_E_CUDA, "second search workspace: %s", cudaGetErrorString(e));
-    h->alt_store_version = h->store_version;
-  }
-  if (!rc)
-    rc = search_core_body(h, q_dev, B, k, out_rows, out_scores, out_keys, stats, robust, async_slot, async_flag_dev, ss);
-  swap_search_ws(h);
-  return rc;
-}
-
-static int search_core_body(rass_engine* h, const float* q_dev, int B, int k, int64_t* out_rows, float* out_scores,
-                            double* out_keys, rass_stats* stats, bool robust, int async_slot, int64_t* async_flag_dev,
-                            cudaStream_t st) {
-  int rc;
-  if ((rc = ensure_query_workspace(h, B))) return rc;
+  if ((rc = ensure_query_workspace(h, ws, B))) return rc;
   rass_stats s;
   memset(&s, 0, sizeof(s));
   s.n_queries = B;
@@ -838,7 +757,7 @@ static int search_core_body(rass_engine* h, const float* q_dev, int B, int k, in
   rass_engine::AsyncSlot* as = async_slot >= 0 ? &h->aslot[async_slot] : nullptr;
   if (as) {
     if (as->pending) return rass_fail(h, RASS_E_INVALID, "async slot %d still has a search in flight", async_slot);
-    if (!as->scal_host) CUDA_TRY(h, cudaMallocHost(&as->scal_host, sizeof(DevScalars)));
+    if (!as->scal_host) CUDA_TRY(h, cudaMallocHost(&as->scal_host, sizeof(SearchScalars)));
     if (!as->done) CUDA_TRY(h, cudaEventCreateWithFlags(&as->done, cudaEventDisableTiming));
   }
   if (h->n_rows == 0) {
@@ -866,28 +785,28 @@ static int search_core_body(rass_engine* h, const float* q_dev, int B, int k, in
   if (robust && path == RASS_PATH_STREAM) path = RASS_PATH_UMMA;    // the streaming scan keeps 32 per warp only
   s.path = path;
   if (!(as && h->async_overlap) && (rc = select_scan_offsets(h, st))) return rc;
-  // (query_prep_kernel resets the per-search device counters; rho_x / max_xnorm stay)
+  // (query_prep_kernel resets the per-search device counters ws.scal)
   if (!as) CUDA_TRY(h, cudaEventRecord(h->ev[0], st));
-  if ((rc = launch_query_prep(h, q_dev, B, st))) return rc;
+  if ((rc = launch_query_prep(h, ws, q_dev, B, st))) return rc;
   s.launches = 1;
   size_t n_ev = 0;
   if (path == RASS_PATH_EXACT) {
-    for (int i = 0; i < B; ++i) h->flagged_host[i] = i;
+    for (int i = 0; i < B; ++i) ws.flagged_host[i] = i;
     CUDA_TRY(h, cudaEventRecord(h->ev[1], st));
-    if ((rc = launch_exact(h, k, h->flagged_host, B, out_rows, out_scores, out_keys, st, &s.launches))) return rc;
+    if ((rc = launch_exact(h, ws, k, ws.flagged_host, B, out_rows, out_scores, out_keys, st, &s.launches))) return rc;
     s.n_fallback = B;
     s.passes = (B + RASS_EXACT_NQ - 1) / RASS_EXACT_NQ;
     s.bytes_streamed = (int64_t)s.passes * h->n_rows * h->dim_pad * ((h->flags & RASS_BF16_ONLY) ? 2 : 4);
   } else if (path == RASS_PATH_GEMM) {
     const int n_segs = scan_gemm_segs(h, B);
     const int seg = robust ? rass_tc_seg(k) : 256;
-    if ((rc = ensure_pool(h, (size_t)n_segs * seg, (size_t)n_segs, (size_t)B))) return rc;
+    if ((rc = ensure_pool(h, ws, (size_t)n_segs * seg, (size_t)n_segs, (size_t)B))) return rc;
     bool cleared = false;
-    if ((rc = launch_seed_thresholds(h, B, seg, (size_t)n_segs * B, &cleared, st))) return rc;
+    if ((rc = launch_seed_thresholds(h, ws, B, seg, (size_t)n_segs * B, &cleared, st))) return rc;
     CUDA_TRY(h, cudaEventRecord(get_event(h, ev_base + n_ev++), st));
-    if ((rc = launch_scan_gemm(h, B, seg, st, cleared))) return rc;
+    if ((rc = launch_scan_gemm(h, ws, B, seg, st, cleared))) return rc;
     CUDA_TRY(h, cudaEventRecord(get_event(h, ev_base + n_ev++), st));
-    if ((rc = launch_finish(h, 0, B, k, n_segs, seg, true, true, out_rows, out_scores, out_keys, st, flag_out)))
+    if ((rc = launch_finish(h, ws, 0, B, k, n_segs, seg, true, true, out_rows, out_scores, out_keys, st, flag_out)))
       return rc;
     s.launches += cleared ? 3 : 4;
     s.passes = (B + 255) / 256;
@@ -896,10 +815,10 @@ static int search_core_body(rass_engine* h, const float* q_dev, int B, int k, in
     const bool umma = path == RASS_PATH_UMMA;
     const int n_segs = umma ? scan_umma_segs(h) : scan_stream_segs(h);
     const int seg = umma ? (robust ? rass_tc_seg(k) : 256) : RASS_STREAM_SEG;
-    if ((rc = ensure_pool(h, (size_t)n_segs * seg, (size_t)n_segs))) return rc;
+    if ((rc = ensure_pool(h, ws, (size_t)n_segs * seg, (size_t)n_segs))) return rc;
     bool cleared = false;
     if (umma) {
-      if ((rc = launch_seed_thresholds(h, B, seg, (size_t)n_segs * RASS_GROUP_Q, &cleared, st))) return rc;
+      if ((rc = launch_seed_thresholds(h, ws, B, seg, (size_t)n_segs * RASS_GROUP_Q, &cleared, st))) return rc;
       s.launches += 1;
     }
     for (int g0 = 0; g0 < B; g0 += RASS_GROUP_Q) {
@@ -907,18 +826,18 @@ static int search_core_body(rass_engine* h, const float* q_dev, int B, int k, in
       CUDA_TRY(h, cudaEventRecord(get_event(h, ev_base + n_ev++), st));
       if (umma) {
         const bool skip_clear = cleared && g0 == 0;      // the seed kernel emptied the pool for the first group
-        if ((rc = launch_scan_umma(h, g0, ng, seg, st, skip_clear))) return rc;
+        if ((rc = launch_scan_umma(h, ws, g0, ng, seg, st, skip_clear))) return rc;
         s.launches += skip_clear ? 1 : 2;
         s.passes += 1;
       } else {
         for (int q0 = g0; q0 < g0 + ng; q0 += 2) {
-          if ((rc = launch_scan_stream(h, q0, std::min(2, g0 + ng - q0), g0, st))) return rc;
+          if ((rc = launch_scan_stream(h, ws, q0, std::min(2, g0 + ng - q0), g0, st))) return rc;
           s.launches += 1;
           s.passes += 1;
         }
       }
       CUDA_TRY(h, cudaEventRecord(get_event(h, ev_base + n_ev++), st));
-      if ((rc = launch_finish(h, g0, ng, k, n_segs, seg, true, umma, out_rows, out_scores, out_keys, st, flag_out)))
+      if ((rc = launch_finish(h, ws, g0, ng, k, n_segs, seg, true, umma, out_rows, out_scores, out_keys, st, flag_out)))
         return rc;
       s.launches += 1;
     }
@@ -926,7 +845,7 @@ static int search_core_body(rass_engine* h, const float* q_dev, int B, int k, in
   }
   if (as) {
     if (path == RASS_PATH_EXACT) return rass_fail(h, RASS_E_INVALID, "the fp64 scan has no async form");
-    CUDA_TRY(h, cudaMemcpyAsync(as->scal_host, h->scal, sizeof(DevScalars), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(h, cudaMemcpyAsync(as->scal_host, ws.scal, sizeof(SearchScalars), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(h, cudaEventRecord(as->done, st));
     as->stats = s;
     as->n_ev = n_ev;
@@ -936,25 +855,21 @@ static int search_core_body(rass_engine* h, const float* q_dev, int B, int k, in
   }
   if (path != RASS_PATH_EXACT) {
     CUDA_TRY(h, cudaEventRecord(h->ev[1], st));
-    CUDA_TRY(h, cudaMemcpyAsync(h->scal_host, h->scal, sizeof(DevScalars), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(h, cudaMemcpyAsync(h->scal_host, ws.scal, sizeof(SearchScalars), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(h, cudaStreamSynchronize(st));
     const int nf = h->scal_host->flagged_n;
     s.n_certified = h->scal_host->n_certified;
     s.max_candidates = h->scal_host->max_cand;
     if (nf > 0) {
-      CUDA_TRY(h, cudaMemcpyAsync(h->flagged_host, h->flagged, (size_t)nf * sizeof(int), cudaMemcpyDeviceToHost, st));
+      CUDA_TRY(h, cudaMemcpyAsync(ws.flagged_host, ws.flagged, (size_t)nf * sizeof(int), cudaMemcpyDeviceToHost, st));
       CUDA_TRY(h, cudaStreamSynchronize(st));
-      std::sort(h->flagged_host, h->flagged_host + nf);
+      std::sort(ws.flagged_host, ws.flagged_host + nf);
       const bool second_chance = !robust && k > 32 && rass_tc_seg(k) != 256;
       if (second_chance) {
         // the recursive search also reuses the timing events: keep this pass's times
         float pre = 0.f;
         CUDA_TRY(h, cudaEventElapsedTime(&pre, h->ev[0], h->ev[1]));
-        for (size_t i = 0; i + 1 < n_ev; i += 2) {
-          float ms1 = 0.f;
-          CUDA_TRY(h, cudaEventElapsedTime(&ms1, h->ev_pool[ev_base + i], h->ev_pool[ev_base + i + 1]));
-          first_scan_ms += ms1;
-        }
+        if ((rc = scan_ms_of(h, ev_base, n_ev, &first_scan_ms))) return rc;
         n_ev = 0;
         first_total_ms = pre;
         // the recursive search reuses every workspace of this one, so stage ids, queries and results on the side
@@ -974,12 +889,12 @@ static int search_core_body(rass_engine* h, const float* q_dev, int B, int k, in
           h->retry_cap = cap;
           h->retry_k = kk;
         }
-        CUDA_TRY(h, cudaMemcpyAsync(h->retry_ids, h->flagged_host, (size_t)nf * sizeof(int), cudaMemcpyHostToDevice, st));
+        CUDA_TRY(h, cudaMemcpyAsync(h->retry_ids, ws.flagged_host, (size_t)nf * sizeof(int), cudaMemcpyHostToDevice, st));
         gather_queries_kernel<<<nf, 256, 0, st>>>(q_dev, h->retry_ids, h->dim, h->retry_q);
         CUDA_TRY(h, cudaGetLastError());
         rass_stats s2;
-        if ((rc = search_core_impl(h, h->retry_q, nf, k, h->retry_rows, h->retry_scores, h->retry_keys, &s2, true, -1,
-                                   nullptr)))
+        if ((rc = search_core_body(h, ws, h->retry_q, nf, k, h->retry_rows, h->retry_scores, h->retry_keys, &s2, true,
+                                   -1, nullptr, st)))
           return rc;
         scatter_results_kernel<<<nf, 128, 0, st>>>(h->retry_ids, k, h->retry_rows, h->retry_scores, h->retry_keys,
                                                    out_rows, out_scores, out_keys);
@@ -993,30 +908,63 @@ static int search_core_body(rass_engine* h, const float* q_dev, int B, int k, in
         retry_scan_ms = s2.scan_ms;
         retry_total_ms = s2.total_ms;
       } else {
-        if ((rc = launch_exact(h, k, h->flagged_host, nf, out_rows, out_scores, out_keys, st, &s.launches))) return rc;
+        if ((rc = launch_exact(h, ws, k, ws.flagged_host, nf, out_rows, out_scores, out_keys, st, &s.launches))) return rc;
         s.n_fallback = nf;
       }
     }
   }
   CUDA_TRY(h, cudaEventRecord(h->ev[2], st));
   CUDA_TRY(h, cudaStreamSynchronize(st));
-  float ms = 0.f;
-  double scan = first_scan_ms;
   if (first_total_ms >= 0.0) {
     s.total_ms = first_total_ms + retry_total_ms;
   } else {
+    float ms = 0.f;
     CUDA_TRY(h, cudaEventElapsedTime(&ms, h->ev[0], h->ev[2]));
     s.total_ms = ms;
   }
-  for (size_t i = 0; i + 1 < n_ev; i += 2) {
-    CUDA_TRY(h, cudaEventElapsedTime(&ms, h->ev_pool[ev_base + i], h->ev_pool[ev_base + i + 1]));
-    scan += ms;
-  }
-  s.scan_ms = scan + retry_scan_ms;
+  double scan = 0.0;
+  if ((rc = scan_ms_of(h, ev_base, n_ev, &scan))) return rc;
+  s.scan_ms = first_scan_ms + scan + retry_scan_ms;
   s.finish_ms = s.total_ms - s.scan_ms;
   h->last_stats = s;
   if (stats) *stats = s;
   return RASS_OK;
+}
+
+int search_core(rass_engine* h, const float* q_dev, int B, int k, int64_t* out_rows, float* out_scores,
+                double* out_keys, rass_stats* stats, int async_slot, int64_t* async_flag_dev) {
+  if (B < 1) return rass_fail(h, RASS_E_INVALID, "B must be >= 1");
+  if (k < 1 || k > RASS_MAX_K) return rass_fail(h, RASS_E_INVALID, "k must be in [1, %d], got %d", RASS_MAX_K, k);
+  // the stream and the workspace of the search: the engine stream and ws[0], except for an async slot under
+  // RASS_OPT_ASYNC_OVERLAP, which runs on its own stream in its own workspace
+  cudaStream_t st = eng_stream(h);
+  SearchWs* ws = &h->ws[0];
+  if (h->async_overlap && async_slot < 0) {
+    // a blocking search shares slot 0's workspace (and must see everything enqueued so far): order it behind the
+    // searches in flight
+    for (auto& a : h->aslot)
+      if (a.pending && a.done) CUDA_TRY(h, cudaStreamWaitEvent(st, a.done, 0));
+  } else if (h->async_overlap) {
+    if (h->aslot[async_slot].pending)
+      return rass_fail(h, RASS_E_INVALID, "async slot %d still has a search in flight", async_slot);
+    if (!h->slot_stream[async_slot]) {
+      CUDA_TRY(h, cudaStreamCreateWithFlags(&h->slot_stream[async_slot], cudaStreamNonBlocking));
+      CUDA_TRY(h, cudaEventCreateWithFlags(&h->slot_fork[async_slot], cudaEventDisableTiming));
+    }
+    // the folded filter offsets are shared by both slots: (re)build them ahead of the fork, on the engine stream
+    const int rc = select_scan_offsets(h, st);
+    if (rc) return rc;
+    CUDA_TRY(h, cudaEventRecord(h->slot_fork[async_slot], st));
+    st = h->slot_stream[async_slot];
+    CUDA_TRY(h, cudaStreamWaitEvent(st, h->slot_fork[async_slot], 0));
+    ws = &h->ws[async_slot];
+    if (!ws->scal) {          // slot 1's workspace, on its first use
+      CUDA_TRY(h, cudaMalloc(&ws->scal, sizeof(SearchScalars)));
+      CUDA_TRY(h, cudaMemsetAsync(ws->scal, 0, sizeof(SearchScalars), st));
+    }
+  }
+  return search_core_body(h, *ws, q_dev, B, k, out_rows, out_scores, out_keys, stats, false, async_slot,
+                          async_flag_dev, st);
 }
 
 extern "C" int rass_search_knn_dev_async(rass_engine* h, const float* q_dev, int B, int k, int64_t* out_rows_dev,
@@ -1026,8 +974,7 @@ extern "C" int rass_search_knn_dev_async(rass_engine* h, const float* q_dev, int
   CHECK_HANDLE(h);
   if (!q_dev || !out_rows_dev || !out_scores_dev) return rass_fail(h, RASS_E_INVALID, "null buffer");
   if (slot < 0 || slot > 1) return rass_fail(h, RASS_E_INVALID, "slot must be 0 or 1");
-  return search_core_impl(h, q_dev, B, k, out_rows_dev, out_scores_dev, out_keys_dev, nullptr, false, slot,
-                          flag_out_dev);
+  return search_core(h, q_dev, B, k, out_rows_dev, out_scores_dev, out_keys_dev, nullptr, slot, flag_out_dev);
 }
 
 extern "C" int rass_search_knn_dev_wait(rass_engine* h, int slot, rass_stats* stats) {
@@ -1044,14 +991,8 @@ extern "C" int rass_search_knn_dev_wait(rass_engine* h, int slot, rass_stats* st
     nf = a.scal_host->flagged_n;
     s.n_certified = a.scal_host->n_certified;
     s.max_candidates = a.scal_host->max_cand;
-    const size_t base = (size_t)1024 * (slot + 1);
-    double scan = 0.0;
-    for (size_t i = 0; i + 1 < a.n_ev; i += 2) {
-      float ms = 0.f;
-      CUDA_TRY(h, cudaEventElapsedTime(&ms, h->ev_pool[base + i], h->ev_pool[base + i + 1]));
-      scan += ms;
-    }
-    s.scan_ms = scan;
+    const int rc = scan_ms_of(h, (size_t)1024 * (slot + 1), a.n_ev, &s.scan_ms);
+    if (rc) return rc;
   }
   s.n_fallback = nf;          // queries whose outputs are NOT final: the caller repeats the search with the blocking call
   if (stats) *stats = s;
@@ -1258,12 +1199,13 @@ extern "C" int rass_debug_gemm_scores(rass_engine* h, const float* q_host, int B
   if (h->n_rows == 0) return RASS_OK;
   int rc;
   float* q_dev = nullptr;
-  if ((rc = ensure_query_workspace(h, B))) return rc;
+  SearchWs& ws = h->ws[0];
+  if ((rc = ensure_query_workspace(h, ws, B))) return rc;
   if ((rc = stage_queries(h, q_host, B, &q_dev))) return rc;
   cudaStream_t st = eng_stream(h);
-  if ((rc = launch_query_prep(h, q_dev, B, st))) return rc;
+  if ((rc = launch_query_prep(h, ws, q_dev, B, st))) return rc;
   if ((rc = select_scan_offsets(h, st))) return rc;
-  return gemm_selftest(h, B, out_host, st);
+  return gemm_selftest(h, ws, B, out_host, st);
 }
 
 extern "C" int rass_debug_umma_scores(rass_engine* h, const float* q_host, int B, float* out_host) {
@@ -1273,10 +1215,11 @@ extern "C" int rass_debug_umma_scores(rass_engine* h, const float* q_host, int B
   if (h->n_rows == 0) return RASS_OK;
   int rc;
   float* q_dev = nullptr;
-  if ((rc = ensure_query_workspace(h, B))) return rc;
+  SearchWs& ws = h->ws[0];
+  if ((rc = ensure_query_workspace(h, ws, B))) return rc;
   if ((rc = stage_queries(h, q_host, B, &q_dev))) return rc;
   cudaStream_t st = eng_stream(h);
-  if ((rc = launch_query_prep(h, q_dev, B, st))) return rc;
+  if ((rc = launch_query_prep(h, ws, q_dev, B, st))) return rc;
   if ((rc = select_scan_offsets(h, st))) return rc;
-  return umma_selftest(h, 0, out_host, st);
+  return umma_selftest(h, ws, 0, out_host, st);
 }

@@ -191,17 +191,18 @@ static int filtered_knn_dev(rass_engine* h, const float* q_dev, int B, int k, co
                             const int64_t* d_rows, size_t max_len, int64_t* out_rows, float* out_scores,
                             double* out_keys, cudaStream_t st) {
   int rc;
-  if ((rc = ensure_query_workspace(h, B))) return rc;
-  if ((rc = launch_query_prep(h, q_dev, B, st))) return rc;
+  SearchWs& ws = h->ws[0];
+  if ((rc = ensure_query_workspace(h, ws, B))) return rc;
+  if ((rc = launch_query_prep(h, ws, q_dev, B, st))) return rc;
   const size_t entries = std::max<size_t>(max_len, 1);
   if ((rc = ensure_xlist_workspace(h, (entries * B + RASS_EXACT_NQ - 1) / RASS_EXACT_NQ))) return rc;
   const size_t smem = (size_t)h->dim_pad * 4;
   if (h->flags & RASS_BF16_ONLY)
-    filtered_keys_kernel<true><<<B, 256, smem, st>>>(h->x32, h->x16, h->norm64, h->sb, h->q_raw, h->q_norm, d_indptr,
+    filtered_keys_kernel<true><<<B, 256, smem, st>>>(h->x32, h->x16, h->norm64, h->sb, ws.q_raw, ws.q_norm, d_indptr,
                                                      d_rows, h->n_rows, h->dim_pad, h->metric, h->xlist_key,
                                                      h->xlist_row, entries);
   else
-    filtered_keys_kernel<false><<<B, 256, smem, st>>>(h->x32, h->x16, h->norm64, h->sb, h->q_raw, h->q_norm, d_indptr,
+    filtered_keys_kernel<false><<<B, 256, smem, st>>>(h->x32, h->x16, h->norm64, h->sb, ws.q_raw, ws.q_norm, d_indptr,
                                                       d_rows, h->n_rows, h->dim_pad, h->metric, h->xlist_key,
                                                       h->xlist_row, entries);
   CUDA_TRY(h, cudaGetLastError());
@@ -271,7 +272,7 @@ extern "C" int rass_search_hybrid_filtered(rass_engine* h, const float* q_host, 
     float* q_dev = nullptr;
     if ((rc = stage_queries(h, q_host, B, &q_dev))) return rc;
     if (knn_mode == 0) {
-      if ((rc = search_core_ex(h, q_dev, B, k, knn_rows, knn_scores, nullptr, &s, -1, nullptr))) return rc;
+      if ((rc = search_core(h, q_dev, B, k, knn_rows, knn_scores, nullptr, &s))) return rc;
     } else {
       if ((rc = filtered_knn_dev(h, q_dev, B, k, d_ip, d_rows, mx, knn_rows, knn_scores, nullptr, st))) return rc;
     }

@@ -30,7 +30,8 @@ struct FinishArgs {
   const float* q_raw;
   const double* q_norm;
   const float* q_rho;       // null when the scan used the fp32 query
-  DevScalars* scal;
+  const StoreScalars* store;   // rho_x, max_xnorm
+  SearchScalars* scal;
   int* flagged;
   int dim_pad, metric, k, g0;
   float acc_eps;
@@ -112,11 +113,11 @@ __global__ void __launch_bounds__(RASS_FINISH_THREADS, 1) finish_kernel(FinishAr
 
   float eps;
   {
-    const float rho_x = BF16_ROWS ? 0.f : a.scal->rho_x;
+    const float rho_x = BF16_ROWS ? 0.f : a.store->rho_x;
     const float rho_q = a.q_rho ? a.q_rho[q] : 0.f;
     float e = rho_x * (1.f + rho_q) + rho_q + a.acc_eps;
     if (a.metric == RASS_METRIC_L2) {
-      const float xm = a.scal->max_xnorm;
+      const float xm = a.store->max_xnorm;
       e = e * xm * (float)a.q_norm[q] * 1.0001f + 6.0e-8f * xm * xm;
     }
     eps = e * 1.0001f;
@@ -209,25 +210,27 @@ static size_t finish_smem(int dim_pad) {
   return (size_t)dim_pad * 4 + RASS_CAND_MAX * 12;
 }
 
-int launch_finish(rass_engine* h, int g0, int ng, int k, int n_segs, int seg_size, bool has_cnt, bool q_is_bf16,
-                  int64_t* out_rows, float* out_scores, double* out_keys, cudaStream_t st, int64_t* flag_out) {
+int launch_finish(rass_engine* h, const SearchWs& ws, int g0, int ng, int k, int n_segs, int seg_size, bool has_cnt,
+                  bool q_is_bf16, int64_t* out_rows, float* out_scores, double* out_keys, cudaStream_t st,
+                  int64_t* flag_out) {
   FinishArgs a;
   a.flag_out = flag_out;
-  a.pool_key = h->pool_key;
-  a.pool_row = h->pool_row;
-  a.pool_thr = h->pool_thr;
-  a.pool_cnt = has_cnt ? h->pool_cnt : nullptr;
-  a.pool_entries = h->pool_entries;
+  a.pool_key = ws.pool_key;
+  a.pool_row = ws.pool_row;
+  a.pool_thr = ws.pool_thr;
+  a.pool_cnt = has_cnt ? ws.pool_cnt : nullptr;
+  a.pool_entries = ws.pool_entries;
   a.n_segs = n_segs;
   a.seg_size = seg_size;
   a.x32 = h->x32;
   a.x16 = h->x16;
   a.norm64 = h->norm64;
-  a.q_raw = h->q_raw;
-  a.q_norm = h->q_norm;
-  a.q_rho = q_is_bf16 ? h->q_rho : nullptr;
-  a.scal = h->scal;
-  a.flagged = h->flagged;
+  a.q_raw = ws.q_raw;
+  a.q_norm = ws.q_norm;
+  a.q_rho = q_is_bf16 ? ws.q_rho : nullptr;
+  a.store = h->store_scal;
+  a.scal = ws.scal;
+  a.flagged = ws.flagged;
   a.dim_pad = h->dim_pad;
   a.metric = h->metric;
   a.k = k;
@@ -414,8 +417,8 @@ __global__ void __launch_bounds__(1024, 1) exact_select_kernel(const double* __r
   }
 }
 
-int launch_exact(rass_engine* h, int k, const int* qids_host, int n_q, int64_t* out_rows, float* out_scores,
-                 double* out_keys, cudaStream_t st, int* launches) {
+int launch_exact(rass_engine* h, const SearchWs& ws, int k, const int* qids_host, int n_q, int64_t* out_rows,
+                 float* out_scores, double* out_keys, cudaStream_t st, int* launches) {
   if (n_q <= 0) return RASS_OK;
   const int M = k <= 32 ? 1 : 4;
   const int grid = h->num_sms * 2;
@@ -426,13 +429,13 @@ int launch_exact(rass_engine* h, int k, const int* qids_host, int n_q, int64_t* 
   const bool bf = (h->flags & RASS_BF16_ONLY) != 0;
   const size_t smem = (size_t)RASS_EXACT_NQ * h->dim_pad * 4;
   // qids live in the (pinned) flagged_host mirror; ship them to the device list
-  int* qids_dev = h->flagged;  // reuse: the flagged list has been consumed by the caller
+  int* qids_dev = ws.flagged;  // reuse: the flagged list has been consumed by the caller
   CUDA_TRY(h, cudaMemcpyAsync(qids_dev, qids_host, (size_t)n_q * sizeof(int), cudaMemcpyHostToDevice, st));
   for (int p = 0; p < n_q; p += RASS_EXACT_NQ) {
     const int nq = n_q - p < RASS_EXACT_NQ ? n_q - p : RASS_EXACT_NQ;
 #define RASS_EX(BF, MM)                                                                                           \
   exact_scan_kernel<BF, MM><<<grid, RASS_WARPS_PER_CTA * 32, smem, st>>>(                                         \
-      h->x32, h->x16, h->norm64, h->sb_scan, h->q_raw, h->q_norm, qids_dev + p, nq, h->n_rows, h->dim_pad, h->metric, \
+      h->x32, h->x16, h->norm64, h->sb_scan, ws.q_raw, ws.q_norm, qids_dev + p, nq, h->n_rows, h->dim_pad, h->metric, \
       h->xlist_key, h->xlist_row, entries)
     if (bf) { if (M == 1) RASS_EX(true, 1); else RASS_EX(true, 4); }
     else    { if (M == 1) RASS_EX(false, 1); else RASS_EX(false, 4); }

@@ -338,35 +338,36 @@ __global__ void clear_gemm_segs_kernel(float* thr, int* cnt, size_t n) {
   cnt[i] = 0;
 }
 
-static int gemm_launch(rass_engine* h, int B, int seg, float* dbg_out, cudaStream_t st, bool pool_cleared = false) {
+static int gemm_launch(rass_engine* h, SearchWs& ws, int B, int seg, float* dbg_out, cudaStream_t st,
+                       bool pool_cleared = false) {
   int rc;
   if (!h->tmap_x) h->tmap_x = calloc(1, sizeof(CUtensorMap));
-  if (!h->tmap_q2) h->tmap_q2 = calloc(1, sizeof(CUtensorMap));
+  if (!ws.tmap_q2) ws.tmap_q2 = calloc(1, sizeof(CUtensorMap));
   if (h->tmap_base != h->x16 || h->tmap_rows != h->cap) {
     if ((rc = encode_rows_map(h, h->tmap_x, h->x16, h->cap, G2_ROWS))) return rc;
     h->tmap_base = h->x16;
     h->tmap_rows = h->cap;
   }
-  if (h->tmap_q2base != h->q16) {
-    if ((rc = encode_rows_map(h, h->tmap_q2, h->q16, h->q_cap, G2_NQ / 2))) return rc;
-    h->tmap_q2base = h->q16;
+  if (ws.tmap_q2base != ws.q16) {
+    if ((rc = encode_rows_map(h, ws.tmap_q2, ws.q16, ws.q_cap, G2_NQ / 2))) return rc;
+    ws.tmap_q2base = ws.q16;
   }
-  if (!h->tmap_q) h->tmap_q = calloc(1, sizeof(CUtensorMap));
-  if (h->tmap_qbase != h->q16) {          // 64-row query boxes: shared with scan_umma, used by the 128-query form
-    if ((rc = encode_rows_map(h, h->tmap_q, h->q16, h->q_cap, 64))) return rc;
-    h->tmap_qbase = h->q16;
+  if (!ws.tmap_q) ws.tmap_q = calloc(1, sizeof(CUtensorMap));
+  if (ws.tmap_qbase != ws.q16) {          // 64-row query boxes: shared with scan_umma, used by the 128-query form
+    if ((rc = encode_rows_map(h, ws.tmap_q, ws.q16, ws.q_cap, 64))) return rc;
+    ws.tmap_qbase = ws.q16;
   }
   const int n_pairs = gemm_pairs(h);
   const GemmPlan plan = make_plan(h, B, n_pairs);
   const int n_segs = scan_gemm_segs(h, B);
   const size_t n = (size_t)n_segs * B;
   if (!pool_cleared) {
-    clear_gemm_segs_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(h->pool_thr, h->pool_cnt, n);
+    clear_gemm_segs_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(ws.pool_thr, ws.pool_cnt, n);
     CUDA_TRY(h, cudaGetLastError());
   }
   // per-query bound shared between the CTAs (ordered-integer image of a float; 0 = nothing published yet): seeded by
   // launch_seed_thresholds before a search; the self-test has no seed
-  if (dbg_out) CUDA_TRY(h, cudaMemsetAsync(h->q_gthr, 0, (size_t)h->q_cap * sizeof(uint32_t), st));
+  if (dbg_out) CUDA_TRY(h, cudaMemsetAsync(ws.q_gthr, 0, (size_t)ws.q_cap * sizeof(uint32_t), st));
   const int grid = 2 * (plan.n_items < n_pairs ? plan.n_items : n_pairs);
   // timing experiments only (results are wrong): 1 = epilogue reads one column block, 2 = epilogue drops every hit
   static const int dbg_mode = getenv("RASS_GEMM_DEBUG_MODE") ? atoi(getenv("RASS_GEMM_DEBUG_MODE")) : 0;
@@ -376,12 +377,12 @@ static int gemm_launch(rass_engine* h, int B, int seg, float* dbg_out, cudaStrea
     CUDA_TRY(h, cudaFuncSetAttribute(scan_gemm_kernel<S, N>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
     scan_gemm_kernel<S, N><<<grid, G2_THREADS, smem, st>>>(                                                          \
         *(CUtensorMap*)h->tmap_x, *(CUtensorMap*)(QMAP), h->sa, h->sb_scan, h->n_rows, plan, h->dim_pad / G2_KBLK,   \
-        B, h->pool_key, h->pool_row, h->pool_thr, h->pool_cnt, h->pool_entries, n_segs, h->q_gthr, dbg_out, dbg_mode); \
+        B, ws.pool_key, ws.pool_row, ws.pool_thr, ws.pool_cnt, ws.pool_entries, n_segs, ws.q_gthr, dbg_out, dbg_mode); \
   } while (0)
   if (gemm_nq(B) == 128) {
-    if (seg == 512) RASS_GEMM_LAUNCH(512, 128, h->tmap_q); else RASS_GEMM_LAUNCH(256, 128, h->tmap_q);
+    if (seg == 512) RASS_GEMM_LAUNCH(512, 128, ws.tmap_q); else RASS_GEMM_LAUNCH(256, 128, ws.tmap_q);
   } else {
-    if (seg == 512) RASS_GEMM_LAUNCH(512, 256, h->tmap_q2); else RASS_GEMM_LAUNCH(256, 256, h->tmap_q2);
+    if (seg == 512) RASS_GEMM_LAUNCH(512, 256, ws.tmap_q2); else RASS_GEMM_LAUNCH(256, 256, ws.tmap_q2);
   }
 #undef RASS_GEMM_LAUNCH
   CUDA_TRY(h, cudaGetLastError());
@@ -390,20 +391,20 @@ static int gemm_launch(rass_engine* h, int B, int seg, float* dbg_out, cudaStrea
 
 // all B prepared queries (q16 rows [0, B), padded with zero rows to a multiple of 256) against the whole shard;
 // query q's candidates land in pool slot q
-int launch_scan_gemm(rass_engine* h, int B, int seg, cudaStream_t st, bool pool_cleared) {
-  return gemm_launch(h, B, seg, nullptr, st, pool_cleared);
+int launch_scan_gemm(rass_engine* h, SearchWs& ws, int B, int seg, cudaStream_t st, bool pool_cleared) {
+  return gemm_launch(h, ws, B, seg, nullptr, st, pool_cleared);
 }
 
 // Debug/self-test entry: raw tensor-core dot products of the first 256 prepared queries against every row.
 // out_host: [n_rows, 256] fp32.
-int gemm_selftest(rass_engine* h, int B, float* out_host, cudaStream_t st) {
+int gemm_selftest(rass_engine* h, SearchWs& ws, int B, float* out_host, cudaStream_t st) {
   float* dbg = nullptr;
   const size_t n = (size_t)h->n_rows * G2_NQ;
   CUDA_TRY(h, cudaMalloc(&dbg, n * 4));
   CUDA_TRY(h, cudaMemsetAsync(dbg, 0, n * 4, st));
   const int n_segs = scan_gemm_segs(h, B);
-  int rc = ensure_pool(h, (size_t)n_segs * 256, (size_t)n_segs, B);
-  if (!rc) rc = gemm_launch(h, B, 256, dbg, st);
+  int rc = ensure_pool(h, ws, (size_t)n_segs * 256, (size_t)n_segs, B);
+  if (!rc) rc = gemm_launch(h, ws, B, 256, dbg, st);
   if (!rc) {
     cudaError_t e = cudaMemcpyAsync(out_host, dbg, n * 4, cudaMemcpyDeviceToHost, st);
     if (e == cudaSuccess) e = cudaStreamSynchronize(st);

@@ -143,15 +143,15 @@ static int stream_ctas(const rass_engine* h) { return h->num_sms * 2; }
 int scan_stream_segs(const rass_engine* h) { return stream_ctas(h); }
 
 template <int NQ>
-static int launch_vec(rass_engine* h, int q0, int slot0, cudaStream_t st) {
+static int launch_vec(rass_engine* h, const SearchWs& ws, int q0, int slot0, cudaStream_t st) {
   const int grid = stream_ctas(h);
   const int n_segs = scan_stream_segs(h);
   const uint4* x = reinterpret_cast<const uint4*>(h->x16);
-  const float* qh = h->q_hat + (size_t)q0 * h->dim_pad;
+  const float* qh = ws.q_hat + (size_t)q0 * h->dim_pad;
 #define RASS_LAUNCH(V)                                                                                          \
-  scan_stream_kernel<NQ, V><<<grid, RASS_WARPS_PER_CTA * 32, 0, st>>>(x, h->sa, h->sb_scan, qh, h->n_rows, h->pool_key, \
-                                                                      h->pool_row, h->pool_thr, h->pool_cnt, slot0, \
-                                                                      n_segs, h->pool_entries)
+  scan_stream_kernel<NQ, V><<<grid, RASS_WARPS_PER_CTA * 32, 0, st>>>(x, h->sa, h->sb_scan, qh, h->n_rows, ws.pool_key, \
+                                                                      ws.pool_row, ws.pool_thr, ws.pool_cnt, slot0, \
+                                                                      n_segs, ws.pool_entries)
   switch (h->dim_pad / 256) {
     case 1: RASS_LAUNCH(1); break;
     case 2: RASS_LAUNCH(2); break;
@@ -164,8 +164,8 @@ static int launch_vec(rass_engine* h, int q0, int slot0, cudaStream_t st) {
   return RASS_OK;
 }
 
-int launch_scan_stream(rass_engine* h, int q0, int nq, int g0, cudaStream_t st) {
-  if (nq == 1) return launch_vec<1>(h, q0, q0 - g0, st);
-  if (nq == 2) return launch_vec<2>(h, q0, q0 - g0, st);
+int launch_scan_stream(rass_engine* h, const SearchWs& ws, int q0, int nq, int g0, cudaStream_t st) {
+  if (nq == 1) return launch_vec<1>(h, ws, q0, q0 - g0, st);
+  if (nq == 2) return launch_vec<2>(h, ws, q0, q0 - g0, st);
   return rass_fail(h, RASS_E_INVALID, "streaming scan takes 1 or 2 queries per pass");
 }

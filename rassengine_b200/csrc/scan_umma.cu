@@ -382,19 +382,19 @@ static void umma_report_times(rass_engine* h, unsigned long long* dbg_t, int gri
           (double)(x_max - t0) * 1e-3);
 }
 
-static int umma_launch(rass_engine* h, int q0, int64_t n_rows, int seg, float* dbg_out, cudaStream_t st) {
+static int umma_launch(rass_engine* h, SearchWs& ws, int q0, int64_t n_rows, int seg, float* dbg_out, cudaStream_t st) {
   int rc;
   if (!h->tmap_x) h->tmap_x = calloc(1, sizeof(CUtensorMap));
-  if (!h->tmap_q) h->tmap_q = calloc(1, sizeof(CUtensorMap));
+  if (!ws.tmap_q) ws.tmap_q = calloc(1, sizeof(CUtensorMap));
   // the map spans the whole reservation (>= 1024 rows); rows >= n_rows are masked in the epilogue
   if (h->tmap_base != h->x16 || h->tmap_rows != h->cap) {
     if ((rc = encode_rows_map(h, (CUtensorMap*)h->tmap_x, h->x16, h->cap, UMMA_ROWS))) return rc;
     h->tmap_base = h->x16;
     h->tmap_rows = h->cap;
   }
-  if (h->tmap_qbase != h->q16) {
-    if ((rc = encode_rows_map(h, (CUtensorMap*)h->tmap_q, h->q16, h->q_cap, UMMA_NQ))) return rc;
-    h->tmap_qbase = h->q16;
+  if (ws.tmap_qbase != ws.q16) {
+    if ((rc = encode_rows_map(h, (CUtensorMap*)ws.tmap_q, ws.q16, ws.q_cap, UMMA_NQ))) return rc;
+    ws.tmap_qbase = ws.q16;
   }
   const int n_tiles = (int)((n_rows + UMMA_ROWS - 1) / UMMA_ROWS);
   // RASS_OPT_SCAN_RESERVE_SMS: leave a few SMs to the kernels that run beside the pass (the other slot's finish, the
@@ -414,9 +414,9 @@ static int umma_launch(rass_engine* h, int q0, int64_t n_rows, int seg, float* d
   do {                                                                                                               \
     CUDA_TRY(h, cudaFuncSetAttribute(scan_umma_kernel<S>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));  \
     scan_umma_kernel<S><<<grid, UMMA_THREADS, smem, st>>>(                                                           \
-        *(CUtensorMap*)h->tmap_x, *(CUtensorMap*)h->tmap_q, h->sa, h->sb_scan, n_rows, n_tiles, h->dim_pad / UMMA_KBLK, \
-        q0, h->pool_key, h->pool_row, h->pool_thr, h->pool_cnt, h->pool_entries, scan_umma_segs(h), h->q_gthr + q0,  \
-        static_tiles ? nullptr : &h->scal->tile_ctr[0], dbg_out, relaxed_wait, dbg_t, umma_stages());                                                                                 \
+        *(CUtensorMap*)h->tmap_x, *(CUtensorMap*)ws.tmap_q, h->sa, h->sb_scan, n_rows, n_tiles, h->dim_pad / UMMA_KBLK, \
+        q0, ws.pool_key, ws.pool_row, ws.pool_thr, ws.pool_cnt, ws.pool_entries, scan_umma_segs(h), ws.q_gthr + q0,  \
+        static_tiles ? nullptr : &ws.scal->tile_ctr[0], dbg_out, relaxed_wait, dbg_t, umma_stages());                                                                                 \
   } while (0)
   if (seg == 512) RASS_UMMA_LAUNCH(512); else RASS_UMMA_LAUNCH(256);
 #undef RASS_UMMA_LAUNCH
@@ -433,30 +433,30 @@ __global__ void clear_segs_kernel(float* thr, int* cnt, size_t n) {
   cnt[i] = 0;
 }
 
-int launch_scan_umma(rass_engine* h, int q0, int nq, int seg, cudaStream_t st, bool pool_cleared) {
+int launch_scan_umma(rass_engine* h, SearchWs& ws, int q0, int nq, int seg, cudaStream_t st, bool pool_cleared) {
   (void)nq;
   if (!pool_cleared) {       // the seed kernel clears for the first group of a search
     const size_t n = (size_t)scan_umma_segs(h) * RASS_GROUP_Q;
-    clear_segs_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(h->pool_thr, h->pool_cnt, n);
+    clear_segs_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(ws.pool_thr, ws.pool_cnt, n);
     CUDA_TRY(h, cudaGetLastError());
   }
-  return umma_launch(h, q0, h->n_rows, seg, nullptr, st);
+  return umma_launch(h, ws, q0, h->n_rows, seg, nullptr, st);
 }
 
 // Debug/self-test entry: raw tensor-core dot products of the first 64 prepared queries against every row.
 // out_host: [n_rows, 64] fp32.  Used by tests to localise descriptor/layout errors.
-int umma_selftest(rass_engine* h, int n_rows_unused, float* out_host, cudaStream_t st) {
+int umma_selftest(rass_engine* h, SearchWs& ws, int n_rows_unused, float* out_host, cudaStream_t st) {
   (void)n_rows_unused;
   float* dbg = nullptr;
   const size_t n = (size_t)h->n_rows * UMMA_NQ;
   CUDA_TRY(h, cudaMalloc(&dbg, n * 4));
   CUDA_TRY(h, cudaMemsetAsync(dbg, 0, n * 4, st));
-  int rc = ensure_pool(h, (size_t)scan_umma_segs(h) * 256, (size_t)scan_umma_segs(h));
+  int rc = ensure_pool(h, ws, (size_t)scan_umma_segs(h) * 256, (size_t)scan_umma_segs(h));
   if (!rc) {
     const size_t ns = (size_t)scan_umma_segs(h) * RASS_GROUP_Q;
-    clear_segs_kernel<<<(unsigned)((ns + 255) / 256), 256, 0, st>>>(h->pool_thr, h->pool_cnt, ns);
-    cudaMemsetAsync(h->q_gthr, 0, UMMA_NQ * sizeof(uint32_t), st);
-    rc = umma_launch(h, 0, h->n_rows, 256, dbg, st);
+    clear_segs_kernel<<<(unsigned)((ns + 255) / 256), 256, 0, st>>>(ws.pool_thr, ws.pool_cnt, ns);
+    cudaMemsetAsync(ws.q_gthr, 0, UMMA_NQ * sizeof(uint32_t), st);
+    rc = umma_launch(h, ws, 0, h->n_rows, 256, dbg, st);
   }
   if (!rc) {
     cudaError_t e = cudaMemcpyAsync(out_host, dbg, n * 4, cudaMemcpyDeviceToHost, st);

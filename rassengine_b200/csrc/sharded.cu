@@ -535,7 +535,7 @@ static int knn_to_coordinator(rass_engine* h, const float* q_host, int B, int k,
     int64_t* o_rows = S->peer_ok || S->dev[g] == h->device ? S->g_rows[0] + (size_t)g * S->cap : S->l_rows[g];
     double* o_keys = S->peer_ok || S->dev[g] == h->device ? S->g_keys[0] + (size_t)g * S->cap : S->l_keys[g];
     // blocking form: certificate failures are retried / re-scanned exactly before it returns (stream synchronised)
-    if ((r = search_core_ex(sh, qd, B, k, o_rows, sh->out_scores, o_keys, &S->st[g], -1, nullptr))) return r;
+    if ((r = search_core(sh, qd, B, k, o_rows, sh->out_scores, o_keys, &S->st[g]))) return r;
     if (o_rows == S->l_rows[g]) {
       cudaError_t e = peer_copy_sync(S->g_rows[0] + (size_t)g * S->cap, h->device, o_rows, S->dev[g], n * 8, eng_stream(sh));
       if (e == cudaSuccess)
@@ -633,7 +633,7 @@ int sharded_search_knn_dev_async(rass_engine* h, const float* q_dev, int B, int 
     double* o_keys = direct ? S->g_keys[slot] + (size_t)g * S->cap : S->l_keys[g];
     int64_t* o_flag = S->g_flag[slot] + g;               // 8 bytes: always a peer store or a small copy below
     int64_t* flag_dst = direct ? o_flag : reinterpret_cast<int64_t*>(sh->out_rows + n);   // spare local word
-    if ((r = search_core_ex(sh, qd, B, k, o_rows, sh->out_scores, o_keys, nullptr, slot, flag_dst))) return r;
+    if ((r = search_core(sh, qd, B, k, o_rows, sh->out_scores, o_keys, nullptr, slot, flag_dst))) return r;
     sg = slot_stream_of(sh, slot);             // RASS_OPT_ASYNC_OVERLAP: the search ran on the slot's own stream
     if (!direct) {
       CUDA_TRY(sh, cudaMemcpyPeerAsync(S->g_rows[slot] + (size_t)g * S->cap, h->device, o_rows, S->dev[g], n * 8, sg));

@@ -13,7 +13,7 @@ __global__ void __launch_bounds__(256) store_convert_kernel(const float* __restr
                                                             int dim_pad, int metric, int bf16_only, int write32,
                                                             float* __restrict__ x32, __nv_bfloat16* __restrict__ x16,
                                                             double* __restrict__ norm64, float* __restrict__ sa,
-                                                            float* __restrict__ sb, DevScalars* scal,
+                                                            float* __restrict__ sb, StoreScalars* scal,
                                                             int64_t first_row, int64_t n) {
   const int lane = threadIdx.x & 31;
   const int64_t r = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
@@ -67,14 +67,13 @@ int launch_store_convert(rass_engine* h, const float* src_dev, int64_t src_strid
                          cudaStream_t st) {
   if (n <= 0) return RASS_OK;
   h->sb_filtered_dirty = true;
-  h->store_version++;
   const bool bf16_only = (h->flags & RASS_BF16_ONLY) != 0;
   const bool in_place = !bf16_only && src_dev == h->x32 + (size_t)first_row * h->dim_pad;
   const int warps = 8;
   int64_t blocks = (n + warps - 1) / warps;
   store_convert_kernel<<<(unsigned)blocks, warps * 32, 0, st>>>(src_dev, src_stride, h->dim, h->dim_pad, h->metric,
                                                                 bf16_only ? 1 : 0, (!bf16_only && !in_place) ? 1 : 0,
-                                                                h->x32, h->x16, h->norm64, h->sa, h->sb, h->scal,
+                                                                h->x32, h->x16, h->norm64, h->sa, h->sb, h->store_scal,
                                                                 first_row, n);
   CUDA_TRY(h, cudaGetLastError());
   return RASS_OK;
@@ -85,10 +84,10 @@ __global__ void __launch_bounds__(128) query_prep_kernel(const float* __restrict
                                                          int B, int B_pad, float* __restrict__ q_raw,
                                                          float* __restrict__ q_hat, __nv_bfloat16* __restrict__ q16,
                                                          double* __restrict__ q_norm, float* __restrict__ q_rho,
-                                                         DevScalars* __restrict__ scal) {
+                                                         SearchScalars* __restrict__ scal) {
   const int lane = threadIdx.x & 31;
   const int b = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-  if (blockIdx.x == 0 && threadIdx.x == 0) {      // the per-search counters (rho_x / max_xnorm stay)
+  if (blockIdx.x == 0 && threadIdx.x == 0) {      // the per-search counters
     scal->flagged_n = 0;
     scal->max_cand = 0;
     scal->n_certified = 0;
@@ -127,12 +126,12 @@ __global__ void __launch_bounds__(128) query_prep_kernel(const float* __restrict
   }
 }
 
-int launch_query_prep(rass_engine* h, const float* q_dev, int B, cudaStream_t st) {
+int launch_query_prep(rass_engine* h, const SearchWs& ws, const float* q_dev, int B, cudaStream_t st) {
   const int B_pad = (B + RASS_QPAD - 1) / RASS_QPAD * RASS_QPAD;
   const int warps = 4;
   query_prep_kernel<<<(B_pad + warps - 1) / warps, warps * 32, 0, st>>>(q_dev, h->dim, h->dim_pad, h->metric, B, B_pad,
-                                                                        h->q_raw, h->q_hat, h->q16, h->q_norm,
-                                                                        h->q_rho, h->scal);
+                                                                        ws.q_raw, ws.q_hat, ws.q16, ws.q_norm,
+                                                                        ws.q_rho, ws.scal);
   CUDA_TRY(h, cudaGetLastError());
   return RASS_OK;
 }
@@ -274,27 +273,28 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(RASS_SEED_THREADS, 1
 // is too small to sample or RASS_DEBUG_NO_SEED is set (the A/B switch of the measurement).  When the kernel runs it
 // also empties the first n_clear segment bounds / sizes of the candidate pool (*cleared = true).  seg = the segment size the
 // scan will use: its compactions keep >= 32 (seg 256) or >= 128 (seg 512) entries above a pivot, and so must the seed.
-int launch_seed_thresholds(rass_engine* h, int B, int seg, size_t n_clear, bool* cleared, cudaStream_t st) {
+int launch_seed_thresholds(rass_engine* h, const SearchWs& ws, int B, int seg, size_t n_clear, bool* cleared,
+                           cudaStream_t st) {
   *cleared = false;
   static const bool no_seed = getenv("RASS_DEBUG_NO_SEED") != nullptr;
   const int B_pad = (B + RASS_QPAD - 1) / RASS_QPAD * RASS_QPAD;
   const int rank = seg == 512 ? 144 : 40;
   if (no_seed || h->n_rows < 16 * RASS_SEED_ROWS) {
-    CUDA_TRY(h, cudaMemsetAsync(h->q_gthr, 0, (size_t)B_pad * sizeof(uint32_t), st));
+    CUDA_TRY(h, cudaMemsetAsync(ws.q_gthr, 0, (size_t)B_pad * sizeof(uint32_t), st));
     return RASS_OK;
   }
   const size_t smem = (size_t)h->dim_pad * sizeof(float) + RASS_SEED_ROWS * sizeof(uint32_t);
   const uint4* x = reinterpret_cast<const uint4*>(h->x16);
   if (h->dim_pad == 1024) {
-    seed_thresholds_kernel<4><<<2 * B_pad, RASS_SEED_THREADS, smem, st>>>(x, h->sa, h->sb_scan, h->q16, h->dim_pad,
-                                                                         h->n_rows, B, rank, h->q_gthr, h->pool_thr,
-                                                                         h->pool_cnt, n_clear);
+    seed_thresholds_kernel<4><<<2 * B_pad, RASS_SEED_THREADS, smem, st>>>(x, h->sa, h->sb_scan, ws.q16, h->dim_pad,
+                                                                         h->n_rows, B, rank, ws.q_gthr, ws.pool_thr,
+                                                                         ws.pool_cnt, n_clear);
   } else {
     if (smem > 48 * 1024)
       CUDA_TRY(h, cudaFuncSetAttribute(seed_thresholds_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    seed_thresholds_kernel<0><<<2 * B_pad, RASS_SEED_THREADS, smem, st>>>(x, h->sa, h->sb_scan, h->q16, h->dim_pad,
-                                                                         h->n_rows, B, rank, h->q_gthr, h->pool_thr,
-                                                                         h->pool_cnt, n_clear);
+    seed_thresholds_kernel<0><<<2 * B_pad, RASS_SEED_THREADS, smem, st>>>(x, h->sa, h->sb_scan, ws.q16, h->dim_pad,
+                                                                         h->n_rows, B, rank, ws.q_gthr, ws.pool_thr,
+                                                                         ws.pool_cnt, n_clear);
   }
   CUDA_TRY(h, cudaGetLastError());
   *cleared = true;

@@ -414,6 +414,65 @@ def test_overlapped_async_slots_equal_the_oracle(path, B, k):
         assert np.array_equal(r, want[1])
 
 
+def _bf16_residual(X, chunk=16384):
+    """||x - bf16(x)|| / ||x|| per row: what store_convert_kernel raises the store's rho_x to."""
+    import torch
+    out = []
+    for i in range(0, X.shape[0], chunk):
+        t = torch.from_numpy(X[i:i + chunk])
+        d = (t - t.to(torch.bfloat16).to(torch.float32)).double()
+        out.append((d.norm(dim=1) / t.double().norm(dim=1)).numpy())
+    return np.concatenate(out)
+
+
+def test_overlapped_async_slots_after_an_append_equal_the_oracle():
+    """RASS_OPT_ASYNC_OVERLAP with an append between overlapped rounds.  Every element of the appended rows sits just
+    below a bf16 rounding midpoint, so their rounding residual is larger than any row's stored before and the store's
+    rho_x (the certificate's allowance for the fp32 rows) rises; they are near copies of the later queries, so they
+    enter those queries' top-k.  Both slots go on after the append, and every batch returns the oracle's ids over the
+    grown corpus."""
+    import torch
+    B, k, n_before, n_batches = 64, 10, 4, 10
+    X = synth.embeddings(150000, 1024, 81)
+    Qs = [synth.embeddings(B, 1024, 82 + i) for i in range(n_batches)]
+    rng = np.random.default_rng(83)
+    later = np.concatenate(Qs[n_before:])
+    block = np.concatenate([later + s / 32 * rng.standard_normal(later.shape, dtype=np.float32) for s in (0.3, 0.5, 0.7)])
+    block = ((block.view(np.uint32) & 0xFFFF0000) | 0x7FFF).view(np.float32)
+    assert _bf16_residual(block).min() > _bf16_residual(X).max()
+    X_all = np.concatenate([X, block])
+    want = [knn.knn_exact(X if i < n_before else X_all, Q, k)[0] for i, Q in enumerate(Qs)]
+    assert all(((w >= X.shape[0]).sum(axis=1) >= 3).all() for w in want[n_before:])
+    with _engine(dim=1024) as e:
+        e.append(X)
+        e.set_async_overlap(True)
+        Qd = [torch.from_numpy(Q).cuda() for Q in Qs]
+        rows = [torch.full((B, k), -7, dtype=torch.int64, device="cuda") for _ in range(2)]
+        scores = [torch.empty((B, k), dtype=torch.float32, device="cuda") for _ in range(2)]
+        flags = [torch.empty(1, dtype=torch.int64, device="cuda") for _ in range(2)]
+        torch.cuda.synchronize()
+        got = [None] * n_batches
+
+        def collect(i):
+            final, st = e.search_knn_dev_wait(i & 1)
+            assert final and int(flags[i & 1].item()) == 0, (i, st)
+            got[i] = rows[i & 1].cpu().numpy().copy()
+
+        for i in range(n_batches):
+            if i == n_before:           # both slots collected, then the append
+                collect(i - 2)
+                collect(i - 1)
+                e.append(block)
+            elif i >= 2 and got[i - 2] is None:
+                collect(i - 2)
+            e.search_knn_dev_async(Qd[i].data_ptr(), B, k, rows[i & 1].data_ptr(), scores[i & 1].data_ptr(), 0, i & 1,
+                                   flags[i & 1].data_ptr())
+        collect(n_batches - 2)
+        collect(n_batches - 1)
+    for i in range(n_batches):
+        assert np.array_equal(got[i], want[i]), i
+
+
 def test_properties_at_2m_rows_all_paths_agree():
     """Larger than the oracle can check in seconds: size-independent properties instead.  On 2M device-generated
     rows every scan path returns the same ids for the same queries, the fp64 scan (the definition) agrees on a
