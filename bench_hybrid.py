@@ -155,7 +155,7 @@ def measure(e, dev, csr, n_docs, B, steps, warmup, n_check, cpu_baseline=True, c
     knn_scores = torch.empty((B, K), dtype=torch.float32, device=dev)
     out_rows = torch.empty((B, K), dtype=torch.int64, device=dev)
     out_scores = torch.empty((B, K), dtype=torch.float32, device=dev)
-    acc = {"scan_ms": 0.0, "text_ms": 0.0, "launches": 0, "n": 0, "order_free": 0}
+    acc = {"scan_ms": 0.0, "text_ms": 0.0, "launches": 0, "n": 0, "order_free": 0, "scan_bytes": 0}
 
     # two batches in flight, like the kNN loop of bench.py: the kNN clause of batch i is enqueued (rass_search_knn_dev_async,
     # its own stream and workspace) before the host turns to the text clauses of batch i-1, so the corpus pass of the
@@ -170,6 +170,7 @@ def measure(e, dev, csr, n_docs, B, steps, warmup, n_check, cpu_baseline=True, c
         if not final:                      # a certificate failed (none on this corpus): the blocking call re-scans
             st = e.search_knn_dev(q_dev[s].data_ptr(), B, K, knn_rows2[slot].data_ptr(), knn_scores2[slot].data_ptr())
         acc["scan_ms"] += st["scan_ms"]
+        acc["scan_bytes"] += st["bytes_streamed"]      # the engine's count: 1 or 2 bytes per element, by the pass it ran
         acc["launches"] += st["launches"]
         e.fuse_hybrid_dev(B, packed[s], W_TEXT, knn_rows2[slot].data_ptr(), knn_scores2[slot].data_ptr(), W_KNN, K,
                           out_rows.data_ptr(), out_scores.data_ptr())
@@ -241,7 +242,8 @@ def measure(e, dev, csr, n_docs, B, steps, warmup, n_check, cpu_baseline=True, c
     res = {"B": B, "k": K, "steps": steps, "warmup": warmup, "ms_dev": ms_dev, "ms_e2e": ms_e2e, "t0": t0, "t1": t1,
            "qps": steps * B / (ms_dev * 1e-3), "qps_e2e": steps * B / (ms_e2e * 1e-3),
            "qps_text_only": steps * B / (ms_text * 1e-3), "qps_one_query_per_call": n_one / (ms_one * 1e-3),
-           "scan_ms": dev_acc["scan_ms"] / max(1, dev_acc["n"]), "text_ms": dev_acc["text_ms"] / max(1, dev_acc["text_n"]),
+           "scan_ms": dev_acc["scan_ms"] / max(1, dev_acc["n"]),
+           "scan_bytes": dev_acc["scan_bytes"] / max(1, dev_acc["n"]), "text_ms": dev_acc["text_ms"] / max(1, dev_acc["text_n"]),
            "text_only_kernel_ms": text_acc["text_ms"] / max(1, text_acc["n"]),
            "launches": int(dev_acc["launches"]), "order_free_batches": int(dev_acc["order_free"]),
            "mean_postings_per_query": float(np.mean(postings)) / B, "postings_per_batch": float(np.mean(postings)),
@@ -303,7 +305,7 @@ def cpu_step_qps(e, idx, qterms, Q, n_docs, B, sample_rows=1_000_000, sample_que
 def roofline_block(res, n_docs):
     import bench
     peak_hbm, _, src = bench.peaks()
-    scan_bytes = n_docs * DIM * 2.0
+    scan_bytes = float(res["scan_bytes"])
     text_bytes = res["postings_per_batch"] * 7.0            # doc id 4 B + tf 2 B + norm byte per posting (SURVEY.md 8d)
     scan = {"kernel": "scan_umma_kernel", "ms": res["scan_ms"], "algorithmic_bytes_per_launch": scan_bytes,
             "achieved_gbs": scan_bytes / (res["scan_ms"] * 1e-3) / 1e9 if res["scan_ms"] else None}

@@ -61,17 +61,24 @@ enum { RASS_METRIC_COSINE = 0, RASS_METRIC_L2 = 1 };
 /* rass_create flags */
 enum {
   RASS_KEEP_FP32 = 1u,  /* resident fp32 matrix + bf16 shadow (default when flags == 0)               */
-  RASS_BF16_ONLY = 2u   /* bf16 corpus: the bf16 values ARE the data (BASELINE config 5, 100M rows)  */
+  RASS_BF16_ONLY = 2u,  /* bf16 corpus: the bf16 values ARE the data (BASELINE config 5, 100M rows)  */
+  RASS_NO_INT8_SHADOW = 4u  /* fp32 store without the int8 shadow (saves dim_pad + 4 bytes per row); the 2..64-query
+                            passes then stream the bf16 shadow.  Alone it still means RASS_KEEP_FP32 */
 };
 
 /* rass_search_* path selection (rass_set_option RASS_OPT_PATH) */
 enum {
-  RASS_PATH_AUTO = 0,    /* B = 1: streaming GEMV+select; B <= 64: tcgen05 tiles, 64 queries per pass;
-                            larger: CTA-pair tcgen05 contraction, 128 (B <= 128) or 256 queries per pass  */
+  RASS_PATH_AUTO = 0,    /* B = 1: streaming GEMV+select; B <= 64: tcgen05 tiles, 64 queries per pass, over the
+                            int8 shadow when the store has one and its quantisation residual is small (else
+                            the bf16 shadow); larger: CTA-pair tcgen05 contraction, 128 (B <= 128) or 256
+                            queries per pass  */
   RASS_PATH_STREAM = 1,  /* force the CUDA-core streaming scan (passes of <= 2 queries)                */
   RASS_PATH_UMMA = 2,    /* force the TMA + tcgen05 scan (passes of <= 64 queries)                     */
   RASS_PATH_EXACT = 3,   /* force the fp64 full scan (the certificate-failure fallback), for tests     */
-  RASS_PATH_GEMM = 4     /* force the CTA-pair (cta_group::2) tcgen05 scan (groups of 256 queries)     */
+  RASS_PATH_GEMM = 4,    /* force the CTA-pair (cta_group::2) tcgen05 scan (groups of 256 queries)     */
+  RASS_PATH_UMMA8 = 5    /* force the TMA + tcgen05 kind::i8 scan over the int8 shadow (passes of <= 64 queries);
+                            queries it cannot certify get the bf16 pass, then the fp64 scan.  RASS_E_UNSUPPORTED on
+                            a store without the int8 shadow */
 };
 
 /* rass_stats.path of a hybrid call: the kNN path in the low byte, plus this bit when the text clauses ran through the
@@ -111,7 +118,7 @@ typedef struct rass_stats {
   int64_t rows_scanned;  /* live + tombstoned rows each pass streams                                   */
   int64_t bytes_streamed;/* algorithmic bytes of the scan passes (rows * dim_pad * sizeof(elem) * passes) */
   int32_t n_queries;
-  int32_t n_certified;   /* queries whose bf16 candidate set was proven to contain the exact top-k     */
+  int32_t n_certified;   /* queries whose scan candidate set was proven to contain the exact top-k     */
   int32_t n_fallback;    /* queries re-scanned exactly in fp64                                         */
   int32_t path;          /* RASS_PATH_* actually used                                                  */
   int32_t passes;        /* corpus passes of the scan                                                  */
@@ -331,6 +338,11 @@ int rass_load(rass_engine* h, const char* path);
 int rass_debug_umma_scores(rass_engine* h, const float* q_host, int B, float* out_host);
 /* same for the CTA-pair kernel: B <= 256 queries, out_host [rows, 256] fp32 */
 int rass_debug_gemm_scores(rass_engine* h, const float* q_host, int B, float* out_host);
+/* same for the int8 pass: the exact int32 accumulators x8 . q8 of B <= 64 queries, acc_host [rows, 128] (columns
+ * 0..63 the first int8 part of each query, 64..127 the second), and the int8 operands the pass read (nullable):
+ * x8_host [rows, dim_pad] and q8_host [128, dim_pad].  RASS_E_UNSUPPORTED on a store without the int8 shadow. */
+int rass_debug_umma8_scores(rass_engine* h, const float* q_host, int B, int32_t* acc_host, int8_t* x8_host,
+                            int8_t* q8_host);
 
 #ifdef __cplusplus
 }

@@ -18,8 +18,8 @@ RASS_E_INVALID, RASS_E_OOM, RASS_E_CUDA, RASS_E_NCCL, RASS_E_NOTFOUND, RASS_E_UN
 ERR_NAMES = {-1: "RASS_E_INVALID", -2: "RASS_E_OOM", -3: "RASS_E_CUDA", -4: "RASS_E_NCCL", -5: "RASS_E_NOTFOUND",
              -6: "RASS_E_UNSUPPORTED", -7: "RASS_E_AGAIN"}
 METRIC_COSINE, METRIC_L2 = 0, 1
-KEEP_FP32, BF16_ONLY = 1, 2
-PATH_AUTO, PATH_STREAM, PATH_UMMA, PATH_EXACT, PATH_GEMM = 0, 1, 2, 3, 4
+KEEP_FP32, BF16_ONLY, NO_INT8_SHADOW = 1, 2, 4
+PATH_AUTO, PATH_STREAM, PATH_UMMA, PATH_EXACT, PATH_GEMM, PATH_UMMA8 = 0, 1, 2, 3, 4, 5
 OPT_PATH, OPT_STREAM, OPT_KNN_PREFILTER, OPT_HYBRID_ORDERED, OPT_HYBRID_MAXSCORE, OPT_ASYNC_OVERLAP, \
     OPT_SCAN_RESERVE_SMS = 1, 2, 3, 4, 5, 6, 7
 PATH_HYBRID_ORDER_FREE = 0x100
@@ -98,6 +98,7 @@ PROTOTYPES = {
     "rass_load": (C.c_int, [_P, C.c_char_p]),
     "rass_debug_umma_scores": (C.c_int, [_P, _P, C.c_int, _P]),
     "rass_debug_gemm_scores": (C.c_int, [_P, _P, C.c_int, _P]),
+    "rass_debug_umma8_scores": (C.c_int, [_P, _P, C.c_int, _P, _P, _P]),
 }
 
 _lib = None

@@ -114,6 +114,7 @@ struct Bm25State {
 struct StoreScalars {
   float rho_x;        // max over rows of ||x - bf16(x)|| / ||x||
   float max_xnorm;    // max over rows of ||x||
+  float rho_x8;       // max over rows of ||x - s_x x8|| / ||x|| (the int8 shadow; 0 without one)
 };
 
 // device-resident counters of one search, reset by query_prep_kernel
@@ -137,6 +138,11 @@ struct SearchWs {
   __nv_bfloat16* q16 = nullptr;     // [q_cap rounded to 64, dim_pad]
   double* q_norm = nullptr;         // [q_cap]
   float* q_rho = nullptr;           // [q_cap] ||q_hat - bf16(q_hat)|| / ||q_hat||
+  // the int8 form of q_hat: q_hat ~ s1 q1 + s2 q2, two int8 parts (the second quantises the first one's residual).
+  // Group g of 64 queries is rows [128 g, 128 g + 128): q1 of its queries, then q2
+  int8_t* q8 = nullptr;             // [q_cap * 2, dim_pad]
+  float* q8_scale = nullptr;        // [q_cap][2] s1, s2
+  float* q_rho8 = nullptr;          // [q_cap] ||q_hat - (s1 q1 + s2 q2)|| / ||q_hat||
   uint32_t* q_gthr = nullptr;       // [q_cap] tcgen05 scans: threshold seed, then the largest pivot any CTA published
   // candidate pool of one query group (RASS_GROUP_Q queries)
   size_t pool_entries = 0;          // per query: stride of the running search
@@ -153,6 +159,8 @@ struct SearchWs {
   void* tmap_q2 = nullptr;          // 128-row boxes (scan_gemm: one CTA's half of a 256-query group)
   const void* tmap_qbase = nullptr; // the q16 each map was encoded for
   const void* tmap_q2base = nullptr;
+  void* tmap_q8 = nullptr;          // over q8, 128-row boxes (scan_umma, int8 pass)
+  const void* tmap_q8base = nullptr;
 };
 
 // a device array that grows in place (vmm.cu): reserved address range, physical chunks mapped on demand
@@ -180,11 +188,20 @@ struct rass_engine {
   double* norm64 = nullptr;         // [cap] ||x|| accumulated in fp64 from the stored values
   float* sa = nullptr;              // [cap] scan scale:  cosine 1/||x|| (0 for zero rows), L2 1
   float* sb = nullptr;              // [cap] scan offset: cosine 0, L2 -0.5||x||^2; -inf = tombstone
-  // the five arrays above live in growable virtual-memory arrays when the driver offers them (vm[i].base == the
+  int8_t* x8 = nullptr;             // [cap, dim_pad] int8 shadow x ~ s_x x8, s_x = max|x| / 127 (null when BF16_ONLY or
+                                    // NO_INT8_SHADOW)
+  float* sa8 = nullptr;             // [cap] scan scale of the int8 shadow: s_x * sa
+  // the seven arrays above live in growable virtual-memory arrays when the driver offers them (vm[i].base == the
   // pointer); otherwise they are cudaMalloc'ed and grow by copy
-  VmArray vm[5];
+  VmArray vm[7];
   bool use_vm = false;
   StoreScalars* store_scal = nullptr;   // device
+  StoreScalars store_scal_host = {};    // host copy, refreshed before a search after rows were written
+  bool store_scal_stale = false;
+  // AUTO takes the int8 64-query pass only for k <= int8_k_max: lowered to k - 1 when an int8 pass AUTO chose left more
+  // than a quarter of a search's queries uncertified (each of those needs the bf16 pass as well, so at that k the bf16
+  // pass alone is cheaper).  The rerank set grows about linearly in k and with the corpus, so it only ever goes down.
+  int int8_k_max = RASS_MAX_K;
   SearchWs ws[2];
   SearchScalars* scal_host = nullptr;   // pinned mirror of ws[0].scal for the blocking search
   cudaStream_t stream = nullptr, user_stream = nullptr, copy_stream = nullptr;
@@ -214,6 +231,9 @@ struct rass_engine {
   void* tmap_x = nullptr;           // host copy of the CUtensorMap over x16 (rebuilt on growth)
   int64_t tmap_rows = -1;
   const void* tmap_base = nullptr;
+  void* tmap_x8 = nullptr;          // the same over x8
+  int64_t tmap8_rows = -1;
+  const void* tmap8_base = nullptr;
   // second-chance pass (queries whose certificate failed at k > 32): ids, gathered queries, results
   int* retry_ids = nullptr;
   float* retry_q = nullptr;
@@ -232,6 +252,7 @@ struct rass_engine {
   // two searches may be in flight through rass_search_knn_dev_async (one slot each)
   struct AsyncSlot {
     bool pending = false, trivial = false;
+    int k = 0;
     SearchScalars* scal_host = nullptr;   // pinned: its own copy, a blocking search may reuse ws[0] before the wait
     cudaEvent_t done = nullptr;
     size_t n_ev = 0;
@@ -275,6 +296,9 @@ static inline cudaStream_t slot_stream_of(const rass_engine* h, int slot) {
 // fp32 accumulation allowance of a length-d dot product with |x||q| <= 1 (gamma_d, doubled for the tensor
 // pipe's unspecified summation order)
 static inline float acc_allowance(int dim_pad) { return (float)dim_pad * 1.1920929e-7f; }
+
+// the store keeps the int8 shadow (x8, sa8)
+static inline bool has_int8_shadow(uint32_t flags) { return !(flags & (RASS_BF16_ONLY | RASS_NO_INT8_SHADOW)); }
 
 // ---------------------------------------------------------------------------------------------
 // device helpers
@@ -488,6 +512,23 @@ __device__ __forceinline__ double exact_key_warp(const float* __restrict__ x32, 
   return -acc;
 }
 
+// Scan key of the int8 pass from the exact integer dots of the row's x8 with the query's two int8 parts: the tcgen05
+// epilogue and the threshold seed both compute it with this one expression (explicitly rounded, never contracted
+// differently), so a seed T is a pivot in the pass's own key units.  |acc| <= 1024 * 127^2 < 2^24: the conversions
+// to float are exact.
+__device__ __forceinline__ float int8_key(int32_t acc1, int32_t acc2, float s1, float s2, float sa8, float sb) {
+  return __fmaf_rn(__fmaf_rn(s1, __int2float_rn(acc1), __fmul_rn(s2, __int2float_rn(acc2))), sa8, sb);
+}
+
+__device__ __forceinline__ float warp_max_nonneg(float v) {
+  return __uint_as_float(__reduce_max_sync(0xffffffffu, __float_as_uint(v)));
+}
+
+// symmetric round-to-nearest int8 code of v at scale s (s = max|.| / 127; 0 codes everything as 0)
+__device__ __forceinline__ float int8_code(float v, float s) {
+  return s > 0.f ? fminf(fmaxf(rintf(__fdiv_rn(v, s)), -127.f), 127.f) : 0.f;
+}
+
 __device__ __forceinline__ float score_from_key(double key, int metric) {
   // OpenSearch k-NN score translation: cosinesimil 1/(2 - cos); l2 1/(1 + d^2)
   return metric == RASS_METRIC_COSINE ? (float)(1.0 / (2.0 - key)) : (float)(1.0 / (1.0 - key));
@@ -502,23 +543,28 @@ int launch_store_convert(rass_engine* h, const float* src_dev, int64_t src_strid
                          cudaStream_t st);
 int launch_query_prep(rass_engine* h, const SearchWs& ws, const float* q_dev, int B, cudaStream_t st);
 int launch_seed_thresholds(rass_engine* h, const SearchWs& ws, int B, int seg, size_t n_clear, bool* cleared,
-                           cudaStream_t st);
+                           cudaStream_t st, bool int8 = false);
 // streaming scan of queries [q0, q0+nq) (nq = 1 or 2); their pool slots are q - g0
 int launch_scan_stream(rass_engine* h, const SearchWs& ws, int q0, int nq, int g0, cudaStream_t st);
 int scan_stream_segs(const rass_engine* h);
-// tcgen05 scan of queries [q0, q0+nq) (nq <= 64) into pool slots 0..nq
-int launch_scan_umma(rass_engine* h, SearchWs& ws, int q0, int nq, int seg, cudaStream_t st, bool pool_cleared = false);
+// tcgen05 scan of queries [q0, q0+nq) (nq <= 64) into pool slots 0..nq; int8: over x8 with the int8 query parts
+int launch_scan_umma(rass_engine* h, SearchWs& ws, int q0, int nq, int seg, cudaStream_t st, bool pool_cleared = false,
+                     bool int8 = false);
 int scan_umma_segs(const rass_engine* h);
 int umma_selftest(rass_engine* h, SearchWs& ws, int n_rows_tile, float* out_host, cudaStream_t st);
+// the int8 pass's raw int32 accumulators of the first 64 prepared queries: out_host [n_rows, 128]
+int umma8_selftest(rass_engine* h, SearchWs& ws, int32_t* out_host, cudaStream_t st);
 // CTA-pair tcgen05 scan of all B prepared queries (groups of 256) into pool slots 0..B
 int launch_scan_gemm(rass_engine* h, SearchWs& ws, int B, int seg, cudaStream_t st, bool pool_cleared = false);
 int scan_gemm_segs(const rass_engine* h, int B);
 int gemm_selftest(rass_engine* h, SearchWs& ws, int B, float* out_host, cudaStream_t st);
-// CUtensorMap over a [rows, dim_pad] bf16 matrix: boxes of box_rows x 64 elements, 128B swizzle
-int encode_rows_map(rass_engine* h, void* map, const void* base, int64_t rows, int box_rows);
+// CUtensorMap over a [rows, dim_pad] bf16 (elem_bytes 2) or int8 (1) matrix: boxes of box_rows x 128 bytes, 128B swizzle
+int encode_rows_map(rass_engine* h, void* map, const void* base, int64_t rows, int box_rows, int elem_bytes = 2);
+// what the scan that filled the pool multiplied: the fp32 query and the stored rows, the bf16 shadows, the int8 ones
+enum ScanOperands { SCAN_FP32_Q = 0, SCAN_BF16 = 1, SCAN_INT8 = 2 };
 // merge the pool of queries [g0, g0+ng), rerank in fp64, emit top-k, flag uncertified queries
 int launch_finish(rass_engine* h, const SearchWs& ws, int g0, int ng, int k, int n_segs, int seg_size, bool has_cnt,
-                  bool q_is_bf16, int64_t* out_rows, float* out_scores, double* out_keys, cudaStream_t st,
+                  ScanOperands ops, int64_t* out_rows, float* out_scores, double* out_keys, cudaStream_t st,
                   int64_t* flag_out = nullptr);
 // fp64 scan of the listed queries (qids host array, n_q of them)
 int launch_exact(rass_engine* h, const SearchWs& ws, int k, const int* qids_host, int n_q, int64_t* out_rows,

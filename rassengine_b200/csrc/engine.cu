@@ -52,18 +52,19 @@ static int ensure_capacity(rass_engine* h, int64_t rows) {
   cudaStream_t st = eng_stream(h);
   const size_t d = (size_t)h->dim_pad;
   const bool bf16_only = (h->flags & RASS_BF16_ONLY) != 0;
-  // bytes per row of x32, x16, norm64, sa, sb
-  const size_t per_row[5] = {bf16_only ? 0 : d * 4, d * 2, 8, 4, 4};
+  const bool int8 = has_int8_shadow(h->flags);
+  // bytes per row of x32, x16, norm64, sa, sb, x8, sa8
+  const size_t per_row[7] = {bf16_only ? 0 : d * 4, d * 2, 8, 4, 4, int8 ? d : 0, int8 ? 4u : 0u};
   if (h->cap == 0 && !h->use_vm && vm_available()) {
     // first allocation: reserve address space for as many rows as the device could ever hold of each array
     size_t free_b = 0, total_b = 0;
     bool ok = cudaMemGetInfo(&free_b, &total_b) == cudaSuccess;
-    for (int i = 0; ok && i < 5; ++i)
+    for (int i = 0; ok && i < 7; ++i)
       if (per_row[i]) {
         const size_t max_rows = std::min<size_t>(0xfffffff0ULL, total_b / per_row[i] + 1);
         ok = vm_reserve(&h->vm[i], h->device, std::max<size_t>(max_rows, (size_t)rows) * per_row[i], 32768 * per_row[i]);
       }
-    if (!ok) for (int i = 0; i < 5; ++i) vm_free(&h->vm[i]);
+    if (!ok) for (int i = 0; i < 7; ++i) vm_free(&h->vm[i]);
     h->use_vm = ok;
   }
   if (h->use_vm) {
@@ -74,7 +75,7 @@ static int ensure_capacity(rass_engine* h, int64_t rows) {
     ncap = std::min<int64_t>(ncap, 0xfffffff0LL);
     for (int pass = 0; pass < 2; ++pass) {
       int bad = 0;
-      for (int i = 0; i < 5 && !bad; ++i)
+      for (int i = 0; i < 7 && !bad; ++i)
         if (per_row[i]) {
           if ((size_t)ncap * per_row[i] > h->vm[i].reserved) ncap = (int64_t)(h->vm[i].reserved / per_row[i]);
           bad = vm_grow(&h->vm[i], (size_t)ncap * per_row[i]);
@@ -88,13 +89,15 @@ static int ensure_capacity(rass_engine* h, int64_t rows) {
     // the capacity in rows is what the smallest mapping holds: chunks are not row-aligned, and the last one mapped is
     // usually only partly asked for
     ncap = 0xfffffff0LL;
-    for (int i = 0; i < 5; ++i)
+    for (int i = 0; i < 7; ++i)
       if (per_row[i]) ncap = std::min<int64_t>(ncap, (int64_t)(h->vm[i].mapped / per_row[i]));
     h->x32 = bf16_only ? nullptr : (float*)h->vm[0].base;
     h->x16 = (__nv_bfloat16*)h->vm[1].base;
     h->norm64 = (double*)h->vm[2].base;
     h->sa = (float*)h->vm[3].base;
     h->sb = (float*)h->vm[4].base;
+    h->x8 = int8 ? (int8_t*)h->vm[5].base : nullptr;
+    h->sa8 = int8 ? (float*)h->vm[6].base : nullptr;
     h->cap = ncap;
     return RASS_OK;
   }
@@ -108,6 +111,10 @@ static int ensure_capacity(rass_engine* h, int64_t rows) {
   if ((rc = dev_realloc(h, &h->norm64, o, n, st))) return rc;
   if ((rc = dev_realloc(h, &h->sa, o, n, st))) return rc;
   if ((rc = dev_realloc(h, &h->sb, o, n, st))) return rc;
+  if (int8) {
+    if ((rc = dev_realloc(h, &h->x8, o * d, n * d, st))) return rc;
+    if ((rc = dev_realloc(h, &h->sa8, o, n, st))) return rc;
+  }
   h->cap = ncap;
   return RASS_OK;
 }
@@ -138,7 +145,7 @@ extern "C" int rass_create(int dim, int metric, int device, int64_t capacity_row
   h->dim_pad = (dim + 255) / 256 * 256;
   h->metric = metric;
   h->device = device;
-  h->flags = flags ? flags : RASS_KEEP_FP32;
+  h->flags = (flags & (RASS_KEEP_FP32 | RASS_BF16_ONLY)) ? flags : flags | RASS_KEEP_FP32;
   h->num_sms = prop.multiProcessorCount;
   auto bail = [&](int code) {
     g_create_error = h->err;
@@ -178,9 +185,10 @@ extern "C" int rass_create(int dim, int metric, int device, int64_t capacity_row
 static void free_search_ws(SearchWs& w) {
   cudaFree(w.scal);
   cudaFree(w.q_raw); cudaFree(w.q_hat); cudaFree(w.q16); cudaFree(w.q_norm); cudaFree(w.q_rho); cudaFree(w.q_gthr);
+  cudaFree(w.q8); cudaFree(w.q8_scale); cudaFree(w.q_rho8);
   cudaFree(w.pool_key); cudaFree(w.pool_row); cudaFree(w.pool_thr); cudaFree(w.pool_cnt);
   cudaFree(w.flagged); cudaFreeHost(w.flagged_host);
-  free(w.tmap_q); free(w.tmap_q2);
+  free(w.tmap_q); free(w.tmap_q2); free(w.tmap_q8);
 }
 
 extern "C" int rass_destroy(rass_engine* h) {
@@ -189,9 +197,10 @@ extern "C" int rass_destroy(rass_engine* h) {
   cudaSetDevice(h->device);
   cudaDeviceSynchronize();
   if (h->use_vm) {
-    for (int i = 0; i < 5; ++i) vm_free(&h->vm[i]);
+    for (int i = 0; i < 7; ++i) vm_free(&h->vm[i]);
   } else {
     cudaFree(h->x32); cudaFree(h->x16); cudaFree(h->norm64); cudaFree(h->sa); cudaFree(h->sb);
+    cudaFree(h->x8); cudaFree(h->sa8);
   }
   cudaFree(h->store_scal); cudaFreeHost(h->scal_host);
   for (SearchWs& w : h->ws) free_search_ws(w);
@@ -223,6 +232,7 @@ extern "C" int rass_destroy(rass_engine* h) {
   cudaFree(b.scratch);
   cudaFree(b.vocab_blob); cudaFree(b.vocab_off); cudaFree(b.fz_terms); cudaFree(b.fz_edits); cudaFree(b.fz_n);
   free(h->tmap_x);
+  free(h->tmap_x8);
   if (h->stream) cudaStreamDestroy(h->stream);
   if (h->copy_stream) cudaStreamDestroy(h->copy_stream);
   delete h;
@@ -243,7 +253,10 @@ extern "C" int rass_set_option(rass_engine* h, int opt, int64_t value) {
       h->bm25.maxscore = value != 0;
       return RASS_OK;
     case RASS_OPT_PATH:
-      if (value < RASS_PATH_AUTO || value > RASS_PATH_GEMM) return rass_fail(h, RASS_E_INVALID, "bad path %lld", (long long)value);
+      if (value < RASS_PATH_AUTO || value > RASS_PATH_UMMA8) return rass_fail(h, RASS_E_INVALID, "bad path %lld", (long long)value);
+      if (value == RASS_PATH_UMMA8 && !has_int8_shadow(h->flags))
+        return rass_fail(h, RASS_E_UNSUPPORTED, "RASS_PATH_UMMA8 needs the int8 shadow (a store without RASS_BF16_ONLY "
+                         "and RASS_NO_INT8_SHADOW)");
       h->path = (int)value;
       return RASS_OK;
     case RASS_OPT_ASYNC_OVERLAP:
@@ -597,11 +610,17 @@ int ensure_query_workspace(rass_engine* h, SearchWs& ws, int B) {
   REALLOC_DEV(h, ws.q_norm, cap);
   REALLOC_DEV(h, ws.q_rho, cap);
   REALLOC_DEV(h, ws.q_gthr, cap);
+  if (has_int8_shadow(h->flags)) {
+    REALLOC_DEV(h, ws.q8, cap * 2 * d);
+    REALLOC_DEV(h, ws.q8_scale, cap * 2);
+    REALLOC_DEV(h, ws.q_rho8, cap);
+  }
   REALLOC_DEV(h, ws.flagged, cap);
   REALLOC_HOST(h, ws.flagged_host, cap);
   ws.q_cap = (int)cap;
   ws.tmap_qbase = nullptr;
   ws.tmap_q2base = nullptr;
+  ws.tmap_q8base = nullptr;
   return RASS_OK;
 }
 
@@ -688,11 +707,41 @@ static int select_scan_offsets(rass_engine* h, cudaStream_t st) {
   return RASS_OK;
 }
 
-static int resolve_path(const rass_engine* h, int B) {
+// Largest rho_x8 for which AUTO scans the int8 shadow.  The int8 certificate allowance is eps ~ rho_x8 + rho_q8
+// (rho_q8 ~ 4e-5 with the two-part query); a query's rerank set holds the pool entries within 2 eps of the k-th best
+// scan key.  Unit rows without outlier channels give rho_x8 ~ 0.014 and ~600 candidates per query at 10M rows x 1024;
+// the count grows faster than linearly in eps (the tail of the score distribution), so 0.03 keeps it below
+// RASS_CAND_MAX = 2048 with room, and the candidate segments keep t + eps below s_k.  Rows with an outlier channel
+// (max|x| far above the rest: s_x = max|x| / 127 quantises everything else coarsely) push rho_x8 past it; the store
+// then keeps the bf16 pass.
+#define RASS_INT8_RHO_MAX 0.03f
+
+// the store facts raised by store_convert_kernel, on the host (appends and overwrites synchronise before they return)
+static int refresh_store_scalars(rass_engine* h) {
+  if (!h->store_scal_stale) return RASS_OK;
+  cudaStream_t st = eng_stream(h);
+  CUDA_TRY(h, cudaMemcpyAsync(&h->store_scal_host, h->store_scal, sizeof(StoreScalars), cudaMemcpyDeviceToHost, st));
+  CUDA_TRY(h, cudaStreamSynchronize(st));
+  h->store_scal_stale = false;
+  return RASS_OK;
+}
+
+static int resolve_path(const rass_engine* h, int B, int k) {
   if (h->path != RASS_PATH_AUTO) return h->path;
   // measured at 10M rows: streaming scan 2.79 ms for one query, 3.10 ms for two; one tcgen05 pass 2.98-3.05 ms for
-  // 1..64 queries; one 256-query CTA-pair pass ~5.1 ms (two 64-query passes = 6.1 ms)
-  return B <= 1 ? RASS_PATH_STREAM : (B <= RASS_GROUP_Q ? RASS_PATH_UMMA : RASS_PATH_GEMM);
+  // 1..64 queries; one 256-query CTA-pair pass ~5.1 ms (two 64-query passes = 6.1 ms).  The int8 pass streams half
+  // the bytes of the bf16 one.  RASS_DEBUG_NO_INT8: the bf16 pass (the A/B switch of the measurement)
+  static const bool no_int8 = getenv("RASS_DEBUG_NO_INT8") != nullptr;
+  if (B <= 1) return RASS_PATH_STREAM;
+  if (B > RASS_GROUP_Q) return RASS_PATH_GEMM;
+  const bool int8 = !no_int8 && h->x8 && h->store_scal_host.rho_x8 <= RASS_INT8_RHO_MAX && k <= h->int8_k_max;
+  return int8 ? RASS_PATH_UMMA8 : RASS_PATH_UMMA;
+}
+
+// after an int8 pass AUTO chose: too many uncertified queries at this k -> the bf16 pass for k and above from now on
+static void note_int8_outcome(rass_engine* h, int path, int B, int k, int n_flagged, bool robust) {
+  if (path == RASS_PATH_UMMA8 && h->path == RASS_PATH_AUTO && !robust && 4 * n_flagged > B)
+    h->int8_k_max = std::min(h->int8_k_max, k - 1);
 }
 
 static cudaEvent_t get_event(rass_engine* h, size_t i) {
@@ -780,9 +829,12 @@ static int search_core_body(rass_engine* h, SearchWs& ws, const float* q_dev, in
     if (stats) *stats = s;
     return RASS_OK;
   }
-  int path = resolve_path(h, B);
+  if ((rc = refresh_store_scalars(h))) return rc;
+  int path = resolve_path(h, B, k);
   int64_t* flag_out = as ? async_flag_dev : nullptr;   // published by the last CTA of the last finish launch
-  if (robust && path == RASS_PATH_STREAM) path = RASS_PATH_UMMA;    // the streaming scan keeps 32 per warp only
+  // the second chance is the bf16 tcgen05 pass: the streaming scan keeps 32 per warp only, and the queries an int8
+  // pass could not certify need the smaller allowance of the bf16 shadow
+  if (robust && (path == RASS_PATH_STREAM || path == RASS_PATH_UMMA8)) path = RASS_PATH_UMMA;
   s.path = path;
   if (!(as && h->async_overlap) && (rc = select_scan_offsets(h, st))) return rc;
   // (query_prep_kernel resets the per-search device counters ws.scal)
@@ -806,19 +858,21 @@ static int search_core_body(rass_engine* h, SearchWs& ws, const float* q_dev, in
     CUDA_TRY(h, cudaEventRecord(get_event(h, ev_base + n_ev++), st));
     if ((rc = launch_scan_gemm(h, ws, B, seg, st, cleared))) return rc;
     CUDA_TRY(h, cudaEventRecord(get_event(h, ev_base + n_ev++), st));
-    if ((rc = launch_finish(h, ws, 0, B, k, n_segs, seg, true, true, out_rows, out_scores, out_keys, st, flag_out)))
+    if ((rc = launch_finish(h, ws, 0, B, k, n_segs, seg, true, SCAN_BF16, out_rows, out_scores, out_keys, st, flag_out)))
       return rc;
     s.launches += cleared ? 3 : 4;
     s.passes = (B + 255) / 256;
     s.bytes_streamed = (int64_t)s.passes * h->n_rows * h->dim_pad * 2;
   } else {
-    const bool umma = path == RASS_PATH_UMMA;
+    const bool int8 = path == RASS_PATH_UMMA8;
+    const bool umma = path == RASS_PATH_UMMA || int8;
+    const ScanOperands ops = int8 ? SCAN_INT8 : (umma ? SCAN_BF16 : SCAN_FP32_Q);
     const int n_segs = umma ? scan_umma_segs(h) : scan_stream_segs(h);
     const int seg = umma ? (robust ? rass_tc_seg(k) : 256) : RASS_STREAM_SEG;
     if ((rc = ensure_pool(h, ws, (size_t)n_segs * seg, (size_t)n_segs))) return rc;
     bool cleared = false;
     if (umma) {
-      if ((rc = launch_seed_thresholds(h, ws, B, seg, (size_t)n_segs * RASS_GROUP_Q, &cleared, st))) return rc;
+      if ((rc = launch_seed_thresholds(h, ws, B, seg, (size_t)n_segs * RASS_GROUP_Q, &cleared, st, int8))) return rc;
       s.launches += 1;
     }
     for (int g0 = 0; g0 < B; g0 += RASS_GROUP_Q) {
@@ -826,7 +880,7 @@ static int search_core_body(rass_engine* h, SearchWs& ws, const float* q_dev, in
       CUDA_TRY(h, cudaEventRecord(get_event(h, ev_base + n_ev++), st));
       if (umma) {
         const bool skip_clear = cleared && g0 == 0;      // the seed kernel emptied the pool for the first group
-        if ((rc = launch_scan_umma(h, ws, g0, ng, seg, st, skip_clear))) return rc;
+        if ((rc = launch_scan_umma(h, ws, g0, ng, seg, st, skip_clear, int8))) return rc;
         s.launches += skip_clear ? 1 : 2;
         s.passes += 1;
       } else {
@@ -837,17 +891,18 @@ static int search_core_body(rass_engine* h, SearchWs& ws, const float* q_dev, in
         }
       }
       CUDA_TRY(h, cudaEventRecord(get_event(h, ev_base + n_ev++), st));
-      if ((rc = launch_finish(h, ws, g0, ng, k, n_segs, seg, true, umma, out_rows, out_scores, out_keys, st, flag_out)))
+      if ((rc = launch_finish(h, ws, g0, ng, k, n_segs, seg, true, ops, out_rows, out_scores, out_keys, st, flag_out)))
         return rc;
       s.launches += 1;
     }
-    s.bytes_streamed = (int64_t)s.passes * h->n_rows * h->dim_pad * 2;
+    s.bytes_streamed = (int64_t)s.passes * h->n_rows * h->dim_pad * (int8 ? 1 : 2);
   }
   if (as) {
     if (path == RASS_PATH_EXACT) return rass_fail(h, RASS_E_INVALID, "the fp64 scan has no async form");
     CUDA_TRY(h, cudaMemcpyAsync(as->scal_host, ws.scal, sizeof(SearchScalars), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(h, cudaEventRecord(as->done, st));
     as->stats = s;
+    as->k = k;
     as->n_ev = n_ev;
     as->trivial = false;
     as->pending = true;
@@ -858,13 +913,15 @@ static int search_core_body(rass_engine* h, SearchWs& ws, const float* q_dev, in
     CUDA_TRY(h, cudaMemcpyAsync(h->scal_host, ws.scal, sizeof(SearchScalars), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(h, cudaStreamSynchronize(st));
     const int nf = h->scal_host->flagged_n;
+    note_int8_outcome(h, s.path, B, k, nf, robust);
     s.n_certified = h->scal_host->n_certified;
     s.max_candidates = h->scal_host->max_cand;
     if (nf > 0) {
       CUDA_TRY(h, cudaMemcpyAsync(ws.flagged_host, ws.flagged, (size_t)nf * sizeof(int), cudaMemcpyDeviceToHost, st));
       CUDA_TRY(h, cudaStreamSynchronize(st));
       std::sort(ws.flagged_host, ws.flagged_host + nf);
-      const bool second_chance = !robust && k > 32 && rass_tc_seg(k) != 256;
+      // k > 32: wider segments; an int8 pass: the bf16 pass (with rass_tc_seg(k) segments)
+      const bool second_chance = !robust && (path == RASS_PATH_UMMA8 || (k > 32 && rass_tc_seg(k) != 256));
       if (second_chance) {
         // the recursive search also reuses the timing events: keep this pass's times
         float pre = 0.f;
@@ -989,6 +1046,7 @@ extern "C" int rass_search_knn_dev_wait(rass_engine* h, int slot, rass_stats* st
   int nf = 0;
   if (!a.trivial) {
     nf = a.scal_host->flagged_n;
+    note_int8_outcome(h, s.path, s.n_queries, a.k, nf, false);
     s.n_certified = a.scal_host->n_certified;
     s.max_candidates = a.scal_host->max_cand;
     const int rc = scan_ms_of(h, (size_t)1024 * (slot + 1), a.n_ev, &s.scan_ms);
@@ -1222,4 +1280,27 @@ extern "C" int rass_debug_umma_scores(rass_engine* h, const float* q_host, int B
   if ((rc = launch_query_prep(h, ws, q_dev, B, st))) return rc;
   if ((rc = select_scan_offsets(h, st))) return rc;
   return umma_selftest(h, ws, 0, out_host, st);
+}
+
+extern "C" int rass_debug_umma8_scores(rass_engine* h, const float* q_host, int B, int32_t* acc_host, int8_t* x8_host,
+                                       int8_t* q8_host) {
+  SHARDED(h, rass_fail(h, RASS_E_UNSUPPORTED, "debug entry points take a single-device handle"));
+  CHECK_HANDLE(h);
+  if (!q_host || !acc_host || B < 1 || B > RASS_GROUP_Q) return rass_fail(h, RASS_E_INVALID, "bad arguments");
+  if (!has_int8_shadow(h->flags)) return rass_fail(h, RASS_E_UNSUPPORTED, "the store has no int8 shadow");
+  if (h->n_rows == 0) return RASS_OK;
+  int rc;
+  float* q_dev = nullptr;
+  SearchWs& ws = h->ws[0];
+  if ((rc = ensure_query_workspace(h, ws, B))) return rc;
+  if ((rc = stage_queries(h, q_host, B, &q_dev))) return rc;
+  cudaStream_t st = eng_stream(h);
+  if ((rc = launch_query_prep(h, ws, q_dev, B, st))) return rc;
+  if ((rc = select_scan_offsets(h, st))) return rc;
+  if ((rc = umma8_selftest(h, ws, acc_host, st))) return rc;
+  const size_t d = (size_t)h->dim_pad;
+  if (x8_host) CUDA_TRY(h, cudaMemcpyAsync(x8_host, h->x8, (size_t)h->n_rows * d, cudaMemcpyDeviceToHost, st));
+  if (q8_host) CUDA_TRY(h, cudaMemcpyAsync(q8_host, ws.q8, 2 * RASS_GROUP_Q * d, cudaMemcpyDeviceToHost, st));
+  CUDA_TRY(h, cudaStreamSynchronize(st));
+  return RASS_OK;
 }

@@ -30,7 +30,8 @@ struct FinishArgs {
   const float* q_raw;
   const double* q_norm;
   const float* q_rho;       // null when the scan used the fp32 query
-  const StoreScalars* store;   // rho_x, max_xnorm
+  const StoreScalars* store;   // rho_x, rho_x8, max_xnorm
+  int int8;                 // the scan read the int8 shadow: rho_x8 bounds its rows (q_rho is then the int8 query's)
   SearchScalars* scal;
   int* flagged;
   int dim_pad, metric, k, g0;
@@ -113,7 +114,7 @@ __global__ void __launch_bounds__(RASS_FINISH_THREADS, 1) finish_kernel(FinishAr
 
   float eps;
   {
-    const float rho_x = BF16_ROWS ? 0.f : a.store->rho_x;
+    const float rho_x = a.int8 ? a.store->rho_x8 : (BF16_ROWS ? 0.f : a.store->rho_x);
     const float rho_q = a.q_rho ? a.q_rho[q] : 0.f;
     float e = rho_x * (1.f + rho_q) + rho_q + a.acc_eps;
     if (a.metric == RASS_METRIC_L2) {
@@ -211,7 +212,7 @@ static size_t finish_smem(int dim_pad) {
 }
 
 int launch_finish(rass_engine* h, const SearchWs& ws, int g0, int ng, int k, int n_segs, int seg_size, bool has_cnt,
-                  bool q_is_bf16, int64_t* out_rows, float* out_scores, double* out_keys, cudaStream_t st,
+                  ScanOperands ops, int64_t* out_rows, float* out_scores, double* out_keys, cudaStream_t st,
                   int64_t* flag_out) {
   FinishArgs a;
   a.flag_out = flag_out;
@@ -227,7 +228,10 @@ int launch_finish(rass_engine* h, const SearchWs& ws, int g0, int ng, int k, int
   a.norm64 = h->norm64;
   a.q_raw = ws.q_raw;
   a.q_norm = ws.q_norm;
-  a.q_rho = q_is_bf16 ? ws.q_rho : nullptr;
+  // acc_eps (below) also covers the int8 pass's fp32 combination s1 * acc1 + s2 * acc2 of exact integer dots: a few
+  // roundings of 2^-24 relative, against dim_pad * 2^-23
+  a.q_rho = ops == SCAN_INT8 ? ws.q_rho8 : (ops == SCAN_BF16 ? ws.q_rho : nullptr);
+  a.int8 = ops == SCAN_INT8;
   a.store = h->store_scal;
   a.scal = ws.scal;
   a.flagged = ws.flagged;

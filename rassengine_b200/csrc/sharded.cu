@@ -236,7 +236,7 @@ extern "C" int rass_create_sharded(int dim, int metric, int n_devices, const int
   h->dim_pad = (dim + 255) / 256 * 256;
   h->metric = metric;
   h->device = device_ids[0];
-  h->flags = flags ? flags : RASS_KEEP_FP32;
+  h->flags = (flags & (RASS_KEEP_FP32 | RASS_BF16_ONLY)) ? flags : flags | RASS_KEEP_FP32;
   S->G = n_devices;
   const int64_t per = capacity_rows > 0 ? (capacity_rows + n_devices - 1) / n_devices + (int64_t(1) << RASS_SHARD_BLOCK_LOG2) : 0;
   for (int g = 0; g < n_devices; ++g) {

@@ -498,6 +498,17 @@ class Engine:
         self._check(self._lib.rass_debug_umma_scores(self._h, _ptr(q), q.shape[0], _ptr(out)))
         return out
 
+    def debug_umma8_scores(self, q: np.ndarray):
+        """The int8 pass's exact int32 accumulators of up to 64 queries against every row, [rows, 128] (column j < 64:
+        x8 . q1 of query j, 64 + j: x8 . q2), with the int8 operands it read: x8 [rows, dim_pad], q8 [128, dim_pad]."""
+        q = np.ascontiguousarray(q, dtype=np.float32).reshape(-1, self.dim)
+        dim_pad = (self.dim + 255) // 256 * 256
+        acc = np.zeros((self.rows(), 128), dtype=np.int32)
+        x8 = np.zeros((self.rows(), dim_pad), dtype=np.int8)
+        q8 = np.zeros((128, dim_pad), dtype=np.int8)
+        self._check(self._lib.rass_debug_umma8_scores(self._h, _ptr(q), q.shape[0], _ptr(acc), _ptr(x8), _ptr(q8)))
+        return acc, x8, q8
+
     def debug_gemm_scores(self, q: np.ndarray) -> np.ndarray:
         """Same through the CTA-pair (cta_group::2) kernel: up to 256 queries, [rows, 256]."""
         q = np.ascontiguousarray(q, dtype=np.float32).reshape(-1, self.dim)
